@@ -40,6 +40,7 @@ import torch  # noqa: E402
 METRIC = "frames/s, 1M Gaussians @1920x1080"
 WORKLOAD = "config3_1m_1080p"
 N_VIEWS = 64
+DUMP_BYTES = 64_000_000  # bound on what --dump-outputs writes
 
 
 def parse_args():
@@ -60,7 +61,16 @@ def parse_args():
     ap.add_argument("--bin-streams", type=int, default=2, help="high-priority binning streams (overlapped pipeline)")
     ap.add_argument("--no-sharded", action="store_true", help="skip the config-4 / config-5 legs (key `sharded`)")
     ap.add_argument("--no-extras", action="store_true", help="skip parity / backward / sharded (quick timing runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the image of the last timed step (rank 0) to DIR/image.npy "
+                         "(float32, H x W x 3; every 2nd row at 4K, to stay within 64 MB): the same arguments "
+                         "render the same inputs, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of the b200 path only")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
@@ -338,6 +348,13 @@ def run_b200(args, rank, world, local_rank):
         assert pipe.check() == 0, "a timed frame overflowed its pair capacity"
     if world > 1:
         dist.barrier()
+    if args.dump_outputs is not None and rank == 0:
+        # what the caller of the pipeline received for step K - 1 (frame k lands in ring slot k % 4); images above
+        # 64 MB (4K) keep every stride-th row so that the dump stays within that size
+        img = ring[(K - 1) % ring.shape[0]]
+        stride = -(-img.numel() * img.element_size() // DUMP_BYTES)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "image.npy"), img[::stride].cpu().numpy())
     total_ms = float(e_beg.elapsed_time(e_end))
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
