@@ -1,5 +1,5 @@
 """compute-sanitizer workload: every kernel of libbsplat.so on small scenes (both rule sets, packed layout, row bands,
-long-list pre-pass, sync-free / captured frames, backward, SH).  Run as
+long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward).  Run as
 
     compute-sanitizer --tool memcheck  python benchmarks/sanitize.py
     compute-sanitizer --tool racecheck python benchmarks/sanitize.py
@@ -66,5 +66,9 @@ for cfg, N, sem in [("config1_1k_256", None, "cuda"), ("config3_1m_1080p", 8000 
     assert torch.equal(rb_img, full)
     coeffs = torch.randn(sc.N, 16, 3, device=dev)
     ms.eval_sh(3, coeffs, g[0], sc.camera)
+    # differentiable frame from the 3D parameters: SH, projection and raster backward
+    p3 = [x.clone().requires_grad_(True) for x in (g[0], g[1], g[2], coeffs)]
+    ms.render_gaussians_diff(p3[0], p3[1], p3[2], g[3], p3[3], sc.camera, sh_degree=3, background_color=bg,
+                             backend=sem).sum().backward()
     torch.cuda.synchronize()
     print(cfg, sem, "ok", float(img.mean()), flush=True)

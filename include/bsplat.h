@@ -26,6 +26,8 @@
  *   bsplat_rasterize_fwd_train / bsplat_rasterize_bwd   no reference counterpart (the reference is
  *                             forward-only: render.py:11 @torch.no_grad, README.md:145); derivative of
  *                             kernels/rasterization.mojo:138-162, checked against torch autograd
+ *   bsplat_project_bwd / bsplat_sh_bwd   no reference counterpart: backward of the projection and of the SH
+ *                             colours (render_gaussians_diff), checked against torch autograd
  *   bsplat_render_fwd         mojosplat/render.py:12-103 render_gaussians (the three stages chained
  *                              on one stream with a single 16-byte read-back)
  *   bsplat_render_enqueue     same without the read-back (device-side M, two-stream overlap, graph capture)
@@ -127,6 +129,19 @@ int bsplat_project_fwd(int64_t N, const float* means3d, const float* log_scales,
                        const float* opacities, const bsplat_camera* cams_host, int32_t n_cams,
                        float eps2d, int32_t semantics, float* means2d, float* conics, float* depths,
                        int32_t* radii, void* stream);
+/* Backward of bsplat_project_fwd for one camera (same eps2d and rule set, no option bits): given the gradients of
+ * the forward's outputs, WRITES (does not accumulate) d loss / d means3d [N,3], d / d log_scales [N,3] and
+ * d / d quats [N,4]; the quaternion gradient is taken with respect to the raw quaternion, through the forward's
+ * normalisation q / max(|q|, 1e-12).  radii is the forward's output: rows with radii == (0, 0) were culled and get
+ * exact zeros (the rasterizer never gives them a gradient; a row behind the camera has infinite intermediates, and
+ * 0 * inf would otherwise turn into NaN).  Clamps follow torch.clamp: the gradient passes through the x/z, y/z clamp of
+ * the Jacobian inside [-lim_neg, lim_pos], bounds included; under BSPLAT_SEM_TORCH no gradient flows through det
+ * where it is clamped at 1e-10.  Opacity only decides the BSPLAT_SEM_GSPLAT radius and cull: no gradient.
+ * v_depths may be NULL (zero).  The forward is recomputed in fp32 from the inputs; nothing is saved by it. */
+int bsplat_project_bwd(int64_t N, const float* means3d, const float* log_scales, const float* quats,
+                       const bsplat_camera* cam_host, float eps2d, int32_t semantics, const int32_t* radii,
+                       const float* v_means2d, const float* v_conics, const float* v_depths, float* v_means3d,
+                       float* v_log_scales, float* v_quats, void* stream);
 
 /* ---- stage 2: binning ---------------------------------------------------------------------- */
 size_t bsplat_bin_scan_workspace_bytes(int64_t N);
@@ -217,6 +232,12 @@ int bsplat_rasterize_stats(int64_t N, int32_t channels, const float* means2d, co
  * campos_host: camera position in world space, 3 floats on the host. */
 int bsplat_sh_eval(int64_t N, int32_t degree, int32_t K_stored, const float* coeffs, const float* means3d,
                    const float* campos_host, float* colors, void* stream);
+/* Backward of bsplat_sh_eval: WRITES v_coeffs [N, K_stored, 3] (= Y_k(dir) v_colors; bands above `degree` are
+ * zero) and, when v_means3d is not NULL, d loss / d means3d [N,3] through dir = normalize(means3d - campos) (zero for
+ * degree 0; the camera gets no gradient).  The clamp max(r + 0.5, 0) passes the gradient like torch.clamp(min=0),
+ * where r + 0.5 >= 0. */
+int bsplat_sh_bwd(int64_t N, int32_t degree, int32_t K_stored, const float* coeffs, const float* means3d,
+                  const float* campos_host, const float* v_colors, float* v_coeffs, float* v_means3d, void* stream);
 
 /* ---- stage 3, training side (SURVEY.md 8f rank 1; the reference is forward-only, render.py:11) --------- */
 /* Forward with the faithful arithmetic (kernels/rasterization.mojo:138-162) that also stores what the

@@ -45,6 +45,7 @@ SYMBOLS = [
     "bsplat_bin2_finish", "bsplat_tile_order", "bsplat_render_begin", "bsplat_render_end",
     "bsplat_render_enqueue", "bsplat_rasterize_workspace_bytes", "bsplat_rasterize_fwd_train",
     "bsplat_rasterize_fwd_train_fast", "bsplat_rasterize_bwd", "bsplat_rasterize_bwd_fast", "bsplat_render_enqueue_band", "bsplat_render_enqueue_band_p2p", "bsplat_sh_eval",
+    "bsplat_project_bwd", "bsplat_sh_bwd",
 ]
 
 
@@ -166,6 +167,10 @@ def load() -> ctypes.CDLL:
                                                      POINTER(c_size_t), c_void_p, c_void_p, c_void_p, c_void_p]
         L.bsplat_sh_eval.argtypes = [c_int64, c_int32, c_int32, c_void_p, c_void_p, POINTER(c_float * 3), c_void_p,
                                      c_void_p]
+        L.bsplat_project_bwd.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, POINTER(BsplatCamera), c_float, c_int32,
+                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
+        L.bsplat_sh_bwd.argtypes = [c_int64, c_int32, c_int32, c_void_p, c_void_p, POINTER(c_float * 3), c_void_p,
+                                    c_void_p, c_void_p, c_void_p]
         L.bsplat_rasterize_stats.argtypes = [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                              c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
                                              c_int32, c_void_p, c_void_p, c_void_p]

@@ -5,6 +5,7 @@ reference's positional order, return arity, shapes and dtypes:
 ``(means2d[N,2] f32, conics[N,3] f32, depths[N] f32, radii[N,2] i32)``.
 New backend strings: ``"cuda"`` (alias ``"b200"``; the reference torch backend's rules,
 projection.py:199-283) and ``"cuda_gsplat"`` (the gsplat / Mojo rules, projection.mojo:59-257).
+``project_gaussians_diff`` is the differentiable form (additive: the reference is forward-only).
 """
 from __future__ import annotations
 
@@ -79,3 +80,48 @@ def project_gaussians_cuda(means3d, scales, quats, opacities, camera, semantics=
                                   _lib.ptr(depths), _lib.ptr(radii), _lib.stream_ptr(dev))
     _lib.check(rc, "bsplat_project_fwd")
     return means2d, conics, depths, radii
+
+
+class _ProjectFn(torch.autograd.Function):
+    """Projection with a backward pass (bsplat_project_fwd / bsplat_project_bwd)."""
+
+    @staticmethod
+    def forward(ctx, means3d, scales, quats, opacities, camera, semantics):
+        means2d, conics, depths, radii = project_gaussians_cuda(means3d, scales, quats, opacities, camera,
+                                                                semantics=semantics)
+        ctx.save_for_backward(_lib.as_f32(means3d, "means3d"), _lib.as_f32(scales, "scales"),
+                              _lib.as_f32(quats, "quats"), radii)
+        ctx.camera, ctx.semantics = camera, semantics
+        ctx.mark_non_differentiable(radii)
+        return means2d, conics, depths, radii
+
+    @staticmethod
+    def backward(ctx, v_means2d, v_conics, v_depths, _v_radii):
+        means3d, scales, quats, radii = ctx.saved_tensors
+        dev = means3d.device
+        L = _lib.require_device(dev)
+        N = means3d.shape[0]
+        v_means2d = _lib.as_f32(v_means2d, "v_means2d")
+        v_conics = _lib.as_f32(v_conics, "v_conics")
+        v_depths = _lib.as_f32(v_depths, "v_depths")
+        v_means3d = torch.empty((N, 3), dtype=torch.float32, device=dev)
+        v_scales = torch.empty((N, 3), dtype=torch.float32, device=dev)
+        v_quats = torch.empty((N, 4), dtype=torch.float32, device=dev)
+        cam = _lib.camera_struct(ctx.camera)
+        with torch.cuda.device(dev):
+            rc = L.bsplat_project_bwd(N, _lib.ptr(means3d), _lib.ptr(scales), _lib.ptr(quats), byref(cam), 0.3,
+                                      ctx.semantics, _lib.ptr(radii), _lib.ptr(v_means2d), _lib.ptr(v_conics),
+                                      _lib.ptr(v_depths), _lib.ptr(v_means3d), _lib.ptr(v_scales), _lib.ptr(v_quats),
+                                      _lib.stream_ptr(dev))
+        _lib.check(rc, "bsplat_project_bwd")
+        return v_means3d, v_scales, v_quats, None, None, None
+
+
+def project_gaussians_diff(means3d, scales, quats, opacities, camera, backend="cuda"):
+    """Differentiable ``project_gaussians`` -> ``(means2d, conics, depths, radii)``.  The forward is the exact stage
+    kernel (values bit-identical to ``project_gaussians``); gradients flow to ``means3d``, the log-``scales`` and the
+    raw (unnormalised) ``quats``.  ``radii`` is not differentiable, and neither is the opacity (it only decides the
+    cull of the ``"cuda_gsplat"`` rules).  Culled rows (radii == 0) get zero gradients."""
+    if backend not in CUDA_BACKENDS:
+        raise ValueError(f"Invalid backend: {backend}")
+    return _ProjectFn.apply(means3d, scales, quats, opacities, camera, CUDA_BACKENDS[backend])

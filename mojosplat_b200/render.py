@@ -6,6 +6,7 @@ intersects :73-76, ``sh_degree`` accepted but only truncating features :82-87). 
 backend the three stages run inside ONE C call (bsplat_render_fwd): projection -> count+scan ->
 one 32-byte read-back (M, depth-key range) -> emit -> onesweep sort -> tile ranges -> raster, all
 on the caller's current stream, workspace reused across frames.
+``render_gaussians_diff`` is the differentiable counterpart (stage by stage, with autograd).
 """
 from __future__ import annotations
 
@@ -15,9 +16,10 @@ from ctypes import byref, c_size_t
 import torch
 
 from . import _lib
-from .binning import bin_gaussians_to_tiles
-from .projection import CUDA_BACKENDS, Camera, project_gaussians
-from .rasterization import RASTER_MODES, rasterize_gaussians
+from .binning import bin_gaussians_to_tiles, bin_gaussians_to_tiles_cuda
+from .projection import CUDA_BACKENDS, Camera, project_gaussians, project_gaussians_diff
+from .rasterization import RASTER_MODES, rasterize_gaussians, rasterize_gaussians_diff
+from .sh import eval_sh_diff
 
 TILE_SIZE = 16
 
@@ -82,6 +84,70 @@ def render_gaussians(
         return torch.zeros(camera.H, camera.W, colors.shape[-1], device=means3d.device, dtype=features.dtype)
     return rasterize_gaussians(means2d, conics, colors, opacities, bg, tile_ranges, sorted_ids, camera,
                                tile_size=tile_size, backend=backend)
+
+
+def render_gaussians_diff(
+    means3d: torch.Tensor,  # (N, 3) world coordinates
+    scales: torch.Tensor,  # (N, 3) log-scales
+    quats: torch.Tensor,  # (N, 4) w,x,y,z, need not be normalised
+    opacities: torch.Tensor,  # (N,) used as given (no activation)
+    features: torch.Tensor,  # (N, C) colours, or (N, K, 3) SH coefficients with sh_degree
+    camera: Camera,
+    sh_degree: int | None = None,
+    background_color: torch.Tensor | None = None,
+    tile_size: int = TILE_SIZE,
+    backend: str = "cuda",
+    return_aux: bool = False,
+):
+    """Differentiable ``render_gaussians``: image (H, W, C) with gradients for means3d, the log-scales, the raw quats,
+    opacities, features (colours or SH coefficients) and a background_color tensor.  Arguments, checks and the
+    features / SH / background rules are those of ``render_gaussians``; the camera gets no gradient.
+
+    Stages: [eval_sh_diff] -> project_gaussians_diff -> binning (the tile lists are constants) ->
+    rasterize_gaussians_diff.  Forward values equal ``render_gaussians``'s for 16x16 tiles and 3 channels; other tile
+    sizes and channel counts (1..4) go through the rasterizer with the reference's operation order.  When no
+    Gaussian overlaps a tile the image is the background (still differentiable with respect to it), where
+    ``render_gaussians`` returns zeros.
+
+    ``return_aux=True`` also returns ``dict(means2d, radii, depths, conics, tile_ranges, sorted_ids)``; ``means2d`` is
+    the tensor of the graph (``retain_grad()`` it for screen-space statistics) and ``radii > 0`` marks the visible
+    Gaussians."""
+    required = [means3d, scales, quats, opacities, features]
+    if not all(isinstance(t, torch.Tensor) and t.is_cuda for t in required):
+        raise ValueError("All input gaussian tensors must be CUDA tensors.")
+    if backend not in CUDA_BACKENDS:
+        raise ValueError(f"Invalid backend: {backend}")
+    if sh_degree is not None and features.dim() == 3:
+        features = eval_sh_diff(int(sh_degree), features, means3d, camera).to(features.dtype)
+        sh_degree = None
+    num_channels = features.shape[-1]
+    bg = _background_tensor(background_color, num_channels, means3d.device, features.dtype)
+    if bg.shape[0] != num_channels:
+        raise ValueError(f"Background color channels ({bg.shape[0]}) must match gaussian color "
+                         f"channels ({num_channels})")
+    assert opacities.shape == (means3d.shape[0],)
+    colors = features
+    if sh_degree is not None:
+        warnings.warn("SH evaluation not implemented; using the first 3 feature channels")
+        if features.shape[-1] > 3:
+            colors = features[..., :3]
+            bg = bg[:3]
+
+    H, W = int(camera.H), int(camera.W)
+    means2d, conics, depths, radii = project_gaussians_diff(means3d, scales, quats, opacities, camera, backend)
+    sorted_ids, tile_ranges = bin_gaussians_to_tiles_cuda(means2d.detach(), radii, depths.detach(), H, W,
+                                                          tile_size, semantics=CUDA_BACKENDS[backend])
+    if sorted_ids.numel() == 0:
+        warnings.warn("No Gaussian overlaps found; returning the background")
+        image = bg.to(torch.float32).expand(H, W, bg.shape[0]).clone()
+    else:
+        image = rasterize_gaussians_diff(means2d, conics, colors, opacities, bg, tile_ranges, sorted_ids, camera,
+                                         tile_size)
+    image = image.to(features.dtype)
+    if return_aux:
+        return image, dict(means2d=means2d, radii=radii, depths=depths, conics=conics, tile_ranges=tile_ranges,
+                           sorted_ids=sorted_ids)
+    return image
 
 
 def _workspace_for(L, dev, N, W, H, tile_size, hint_M=None):
