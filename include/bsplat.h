@@ -77,7 +77,6 @@ extern "C" {
 #define BSPLAT_RASTER_FAST_NOCULL 2  /* fast arithmetic without sub-tile culling (exactness A/B) */
 
 /* bsplat_render_fwd `flags`: low byte = rasterizer mode, plus */
-#define BSPLAT_FLAG_BIN_SINGLE_LEVEL 0x100  /* one sort of packed 64-bit keys instead of the two-level sort */
 #define BSPLAT_FLAG_CAMERA_INDIRECT 0x200   /* bsplat_render_enqueue: the camera pose / intrinsics are read
                                                from `cam` (pinned host memory) when the stream gets there, so a
                                                captured CUDA graph can be replayed with a new pose; width and
@@ -87,11 +86,9 @@ extern "C" {
                                                sort, count + scan and the raster records only see the visible ones
                                                (projection.mojo:73-87,213-244; gsplat packed=True).  Same image and
                                                lists.  A no-op under BSPLAT_SEM_TORCH, where every Gaussian owns a tile */
-#define BSPLAT_FLAG_PROJ_FMA 0x800          /* the BSPLAT_PROJ_ALLOW_FMA projection inside a fused frame */
 #define BSPLAT_FLAG_NO_BAND_PRETEST 0x1000  /* row-band frames: project every Gaussian instead of only those a
                                              * conservative pre-test cannot rule out of the band (A/B and tests:
                                              * both ways give bit-identical lists and images) */
-#define BSPLAT_FLAG_PROJ_FAST 0x2000        /* the BSPLAT_PROJ_FAST_MATH projection inside a fused frame */
 
 /* Pinhole camera, world->camera. Mirrors mojosplat/utils.py:5-31 (Camera.view_matrix, Ks, H, W,
  * near, far) as a POD. viewmat is row-major 4x4. */
@@ -304,7 +301,7 @@ int bsplat_render_fwd(int64_t N, const float* means3d, const float* log_scales, 
  * and an ASYNC copy of the bin info (M) into pinned host memory -- no sync. The caller waits for the
  * stream (event), reads M, then calls end (emit + tile sort + ranges + raster) with the same workspace,
  * which must hold bsplat_render_workspace_bytes(N, M, ...). Two streams with one workspace each overlap
- * begin(k+1) with end(k). Two-level binning only. */
+ * begin(k+1) with end(k). */
 int bsplat_render_begin(int64_t N, const float* means3d, const float* log_scales, const float* quats,
                         const float* opacities, const bsplat_camera* cam_host, int32_t tile_size,
                         int32_t semantics, void* workspace, size_t workspace_bytes,

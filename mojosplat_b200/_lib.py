@@ -24,14 +24,11 @@ OK = 0
 E_ARG, E_WORKSPACE, E_OVERFLOW, E_NODEVICE = -1, -2, -3, -4
 SEM_TORCH, SEM_GSPLAT = 0, 1
 RASTER_FAST, RASTER_FAITHFUL, RASTER_FAST_NOCULL = 0, 1, 2
-FLAG_BIN_SINGLE_LEVEL = 0x100
 FLAG_CAMERA_INDIRECT = 0x200
 FLAG_PACKED = 0x400
-FLAG_PROJ_FMA = 0x800
 FLAG_NO_BAND_PRETEST = 0x1000
 PROJ_ALLOW_FMA = 0x100  # or-ed into `semantics` of bsplat_project_fwd
 PROJ_FAST_MATH = 0x200  # ditto: the "within 1e-4" build (radii may be one off at integer boundaries)
-FLAG_PROJ_FAST = 0x2000
 BIN_PACKED = 0x100      # or-ed into `semantics` of bsplat_bin2_prepare / bsplat_bin2_finish
 
 # every symbol include/bsplat.h declares (checked by tests/test_capi_symbols.py)

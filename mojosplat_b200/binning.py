@@ -37,7 +37,8 @@ def bin_gaussians_to_tiles(
 
 
 def read_bin_info(info_dev: torch.Tensor) -> _lib.BsplatBinInfo:
-    """The single device->host read-back of the stage (32 bytes: M and the depth-key range)."""
+    """A bin info (32 bytes: M, the depth-key range, the overflow flag) from a device tensor -- the single device->host
+    read-back of the stage -- or from a host block (no copy)."""
     host = info_dev.cpu().numpy().tobytes()
     return _lib.BsplatBinInfo.from_buffer_copy(host)
 

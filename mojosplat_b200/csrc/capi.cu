@@ -21,9 +21,6 @@ int project_fwd_launch(int64_t N, const float* means3d, const float* log_scales,
                        const float* opacities, const bsplat_camera& cam, float eps2d, int semantics,
                        float* means2d, float* conics, float* depths, int32_t* radii, cudaStream_t stream,
                        const bsplat_camera* cam_dev, const ProjExtra* extra, int variant);
-inline int proj_variant_of(int flags) {
-    return (flags & BSPLAT_FLAG_PROJ_FAST) ? 2 : ((flags & BSPLAT_FLAG_PROJ_FMA) ? 1 : 0);
-}
 int rasterize_launch(int64_t N, int channels, const float* means2d, const float* conics, const float* colors,
                      const float* opacities, const float* background_dev, const int32_t* tile_ranges,
                      const int32_t* tile_order, const int32_t* sorted_ids, int W, int H, int tile_size,
@@ -119,34 +116,6 @@ namespace {
 constexpr size_t kAlign = 256;
 inline size_t align_up(size_t v) { return (v + kAlign - 1) / kAlign * kAlign; }
 
-// single-level binning scratch (BSPLAT_FLAG_BIN_SINGLE_LEVEL)
-struct Bin1Ws {
-    uint32_t* offsets; bsplat_bin_info* info; void* scan_ws; size_t scan_bytes;
-    uint64_t* keys; uint64_t* keys_alt; int32_t* ids; int32_t* ids_alt;
-    void* sort_ws; size_t sort_bytes;
-    size_t total;
-};
-
-Bin1Ws carve_bin1(void* base, int64_t N, int64_t M) {
-    Bin1Ws w;
-    char* p = static_cast<char*>(base);
-    size_t off = 0;
-    auto take = [&](size_t bytes) { void* r = p ? p + off : nullptr; off += align_up(bytes); return r; };
-    const size_t n = (size_t)(N > 0 ? N : 1), m = (size_t)(M > 0 ? M : 1);
-    w.offsets = (uint32_t*)take((n + 1) * sizeof(uint32_t));
-    w.info = (bsplat_bin_info*)take(sizeof(bsplat_bin_info));
-    w.scan_bytes = bsplat_bin_scan_workspace_bytes(N);
-    w.scan_ws = take(w.scan_bytes);
-    w.keys = (uint64_t*)take(m * sizeof(uint64_t));
-    w.keys_alt = (uint64_t*)take(m * sizeof(uint64_t));
-    w.ids = (int32_t*)take(m * sizeof(int32_t));
-    w.ids_alt = (int32_t*)take(m * sizeof(int32_t));
-    w.sort_bytes = bsplat_radix_sort_workspace_bytes(M, 0, 64);
-    w.sort_ws = take(w.sort_bytes);
-    w.total = off;
-    return w;
-}
-
 struct RenderWs {
     float* means2d; float* conics; float* depths; int32_t* radii;
     int32_t* tile_ranges; int32_t* tile_order; int32_t* sorted_ids;
@@ -158,7 +127,7 @@ struct RenderWs {
     size_t total;
 };
 
-RenderWs carve_render(void* base, int64_t N, int64_t M, int W, int H, int tile_size, bool single_level) {
+RenderWs carve_render(void* base, int64_t N, int64_t M, int W, int H, int tile_size) {
     RenderWs w;
     char* p = static_cast<char*>(base);
     size_t off = 0;
@@ -174,7 +143,7 @@ RenderWs carve_render(void* base, int64_t N, int64_t M, int W, int H, int tile_s
     w.cam_dev = (bsplat_camera*)take(sizeof(bsplat_camera));
     w.raster_rec = take(raster_workspace_bytes(N));
     // the N-dependent part of the binning scratch comes first so that it survives the re-carve with M
-    w.bin_bytes = single_level ? carve_bin1(nullptr, N, M).total : bin2_workspace_bytes(N, M, (int64_t)tiles_w * tiles_h);
+    w.bin_bytes = bin2_workspace_bytes(N, M, (int64_t)tiles_w * tiles_h);
     w.bin_ws = take(w.bin_bytes);
     w.sorted_ids = (int32_t*)take(m * sizeof(int32_t));
     w.long_surv = (int32_t*)take(raster_long_surv_bytes(M));
@@ -183,9 +152,38 @@ RenderWs carve_render(void* base, int64_t N, int64_t M, int W, int H, int tile_s
     return w;
 }
 
-inline bool fast_raster_for(int raster_mode, int tile_size, int channels) {
-    return (raster_mode == BSPLAT_RASTER_FAST || raster_mode == BSPLAT_RASTER_FAST_NOCULL) && tile_size == 16 &&
-           channels == 3;
+// The arguments of a fused frame after the checks every frame entry point shares, and what follows from them.  Each
+// entry point adds its own rules (N > 0, M, streams, which Gaussian arrays must be present).
+struct Frame {
+    int64_t N;
+    const float *means3d, *log_scales, *quats, *opacities, *colors, *background;
+    float* image;
+    const bsplat_camera* cam;
+    int channels, tile_size, semantics, flags, raster_mode;
+    bool fast_raster;  // the fast kernel with raster records and the longest-first tile order (16x16 tiles, RGB)
+    int W, H, tiles_w, tiles_h;
+    int row0, row1;    // tile rows that are binned and rasterized: all of them unless a band entry narrows them
+};
+
+int make_frame(int64_t N, const float* means3d, const float* log_scales, const float* quats, const float* opacities,
+               const float* colors, int channels, const bsplat_camera* cam, const float* background, int tile_size,
+               int semantics, int flags, float* image, Frame* f) {
+    if (!cam || N < 0 || tile_size <= 0 || tile_size > 32) return BSPLAT_E_ARG;
+    if (semantics != BSPLAT_SEM_TORCH && semantics != BSPLAT_SEM_GSPLAT) return BSPLAT_E_ARG;
+    if (cam->width <= 0 || cam->height <= 0) return BSPLAT_E_ARG;
+    f->N = N;
+    f->means3d = means3d; f->log_scales = log_scales; f->quats = quats; f->opacities = opacities;
+    f->colors = colors; f->background = background; f->image = image;
+    f->cam = cam;
+    f->channels = channels; f->tile_size = tile_size; f->semantics = semantics; f->flags = flags;
+    f->raster_mode = flags & 0xff;
+    f->fast_raster = (f->raster_mode == BSPLAT_RASTER_FAST || f->raster_mode == BSPLAT_RASTER_FAST_NOCULL) &&
+                     tile_size == 16 && channels == 3;
+    f->W = cam->width; f->H = cam->height;
+    f->tiles_w = (f->W + tile_size - 1) / tile_size;
+    f->tiles_h = (f->H + tile_size - 1) / tile_size;
+    f->row0 = 0; f->row1 = f->tiles_h;
+    return BSPLAT_OK;
 }
 
 // CUDA events of the per-stage timing; destroyed on every exit path
@@ -207,46 +205,96 @@ struct StageEvents {
     }
 };
 
-// Front half of a two-level frame: control words zeroed, projection with the fused epilogue (tile rectangles, depth
-// keys + histograms, raster records), [compaction,] depth sort, count + scan.  write_stage_outputs: also store the
-// reference's four projection outputs (needed by the faithful rasterizer, the aux outputs and nobody else).
-int frame_front(int64_t N, const float* means3d, const float* log_scales, const float* quats, const float* opacities,
-                const float* colors, const bsplat_camera& cam, const bsplat_camera* cam_dev, int tile_size,
-                int semantics, int flags, int row0, int row1, bool want_rec, float* o_means2d, float* o_conics,
+// Front half of a frame: control words zeroed, projection with the fused epilogue (tile rectangles, depth keys +
+// histograms, raster records), [compaction,] depth sort, count + scan.  o_*: also store the reference's four projection
+// outputs (needed by the faithful rasterizer, the aux outputs and nobody else); nullptr skips them.
+int frame_front(const Frame& f, const bsplat_camera* cam_dev, bool want_rec, float* o_means2d, float* o_conics,
                 float* o_depths, int32_t* o_radii, const RenderWs& w, cudaStream_t stream,
                 cudaEvent_t ev_after_projection = nullptr) {
-    const int W = cam.width, H = cam.height;
     BinParams p;
-    int rc = make_bin_params(W, H, tile_size, row0, row1, semantics, &p);
+    int rc = make_bin_params(f.W, f.H, f.tile_size, f.row0, f.row1, f.semantics, &p);
     if (rc != BSPLAT_OK) return rc;
-    const bool compact = (flags & BSPLAT_FLAG_PACKED) != 0 || p.row_begin > 0 || p.row_end < p.tiles_h;
-    rc = bin2_begin(N, w.bin_ws, w.bin_bytes, stream);
+    const bool compact = (f.flags & BSPLAT_FLAG_PACKED) != 0 || p.row_begin > 0 || p.row_end < p.tiles_h;
+    rc = bin2_begin(f.N, w.bin_ws, w.bin_bytes, stream);
     if (rc != BSPLAT_OK) return rc;
     ProjExtra ex;
-    bin2_prep_targets(w.bin_ws, N, compact, &ex.rects, &ex.dkeys, &ex.hist);
+    bin2_prep_targets(w.bin_ws, f.N, compact, &ex.rects, &ex.dkeys, &ex.hist);
     ex.rec = want_rec ? w.raster_rec : nullptr;
-    ex.colors = colors;
-    ex.opac = opacities;
-    ex.tile_size = tile_size;
+    ex.colors = f.colors;
+    ex.opac = f.opacities;
+    ex.tile_size = f.tile_size;
     ex.rec_row_begin = p.row_begin;
     ex.rec_row_end = p.row_end;
     // Row bands under the torch rules (and nobody asking for the stage outputs): a cheap conservative pre-test on
     // the raw inputs first lists the Gaussians whose rectangle can reach the band at all; only those are projected
     // and compacted.  (What every rank of a band split repeats shrinks from all N to its candidates.)
     const bool band = p.row_begin > 0 || p.row_end < p.tiles_h;
-    const bool pretest = band && semantics == BSPLAT_SEM_TORCH && cam_dev == nullptr && o_means2d == nullptr &&
-                         (flags & BSPLAT_FLAG_NO_BAND_PRETEST) == 0 && N > 0;
+    const bool pretest = band && f.semantics == BSPLAT_SEM_TORCH && cam_dev == nullptr && o_means2d == nullptr &&
+                         (f.flags & BSPLAT_FLAG_NO_BAND_PRETEST) == 0 && f.N > 0;
     if (pretest) {
-        rc = bin2_band_candidates(N, means3d, log_scales, cam, 0.3f, p, w.bin_ws, w.bin_bytes, stream, &ex.list,
-                                  &ex.list_n);
+        rc = bin2_band_candidates(f.N, f.means3d, f.log_scales, *f.cam, 0.3f, p, w.bin_ws, w.bin_bytes, stream,
+                                  &ex.list, &ex.list_n);
         if (rc != BSPLAT_OK) return rc;
     }
-    rc = project_fwd_launch(N, means3d, log_scales, quats, opacities, cam, 0.3f, semantics, o_means2d, o_conics,
-                            o_depths, o_radii, stream, cam_dev, &ex, proj_variant_of(flags));
+    rc = project_fwd_launch(f.N, f.means3d, f.log_scales, f.quats, f.opacities, *f.cam, 0.3f, f.semantics, o_means2d,
+                            o_conics, o_depths, o_radii, stream, cam_dev, &ex, 0);
     if (rc != BSPLAT_OK) return rc;
     if (ev_after_projection) BSPLAT_CUDA_TRY(cudaEventRecord(ev_after_projection, stream));
-    return bin2_prepare(N, nullptr, nullptr, 0, nullptr, p, w.bin_ws, w.bin_bytes, stream, /*have_prep=*/true, compact,
+    return bin2_prepare(f.N, nullptr, nullptr, 0, nullptr, p, w.bin_ws, w.bin_bytes, stream, /*have_prep=*/true, compact,
                         pretest);
+}
+
+// Back half of a frame: emission, tile sort, tile ranges and tile order (bin2_finish), then the rasterizer.
+// M is the pair count the caller read back or, with device_m, the capacity of the pair buffers (the real count stays on
+// the device).  Binning runs on sb, the rasterizer on sr; when they differ, event_bin_done orders the two.
+// rec_ready: the front half built the raster records.  info_host (nullable): pinned host block that receives the frame's
+// bin info.  te (nullable): stage-timing marks 2 (before the emission) and 3 (before the rasterizer).
+int frame_back(const Frame& f, const RenderWs& w, int64_t M, bool device_m, const float* means2d, const float* conics,
+               int32_t* tile_ranges, bool rec_ready, const PeerImages* peers, cudaStream_t sb, cudaStream_t sr,
+               cudaEvent_t event_bin_done, bsplat_bin_info* info_host, StageEvents* te) {
+    BinParams p;
+    int rc = make_bin_params(f.W, f.H, f.tile_size, f.row0, f.row1, f.semantics, &p);
+    if (rc != BSPLAT_OK) return rc;
+    if (te && (rc = te->record(2, sb)) != BSPLAT_OK) return rc;
+    // the bin info reaches the host as a store from the last binning kernel when the block is device-accessible
+    // (pinned memory under UVA); a copy-engine transfer would queue behind image downloads of earlier frames
+    bool info_direct = false;
+    if (info_host) {
+        cudaPointerAttributes attr;
+        if (cudaPointerGetAttributes(&attr, info_host) == cudaSuccess && attr.type == cudaMemoryTypeHost &&
+            attr.devicePointer == (void*)info_host)
+            info_direct = true;
+        else
+            (void)cudaGetLastError();
+    }
+    rc = bin2_finish(f.N, M, device_m, p, w.bin_ws, w.bin_bytes, w.sorted_ids, tile_ranges, w.tile_order, sb,
+                     (f.flags & BSPLAT_FLAG_PACKED) != 0, info_direct ? info_host : nullptr);
+    if (rc != BSPLAT_OK) return rc;
+    const bsplat_bin_info* d_info = bin2_info_ptr(w.bin_ws, f.N);
+    if (info_host && !info_direct)
+        BSPLAT_CUDA_TRY(cudaMemcpyAsync(info_host, d_info, sizeof(bsplat_bin_info), cudaMemcpyDeviceToHost, sb));
+    if (sr != sb) {
+        BSPLAT_CUDA_TRY(cudaEventRecord(event_bin_done, sb));
+        BSPLAT_CUDA_TRY(cudaStreamWaitEvent(sr, event_bin_done, 0));
+    }
+    const unsigned long long* m_dev = nullptr;
+    if (device_m) {
+        // "no intersections at all => all-zero image" (render.py:73-76) is a whole-frame rule: a partial band decides
+        // it from the number of Gaussians that own a tile anywhere in the frame (counted by the compaction pass)
+        m_dev = reinterpret_cast<const unsigned long long*>(d_info);
+        if (f.row0 > 0 || f.row1 < f.tiles_h) {
+            const int32_t* perm;
+            const unsigned long long* n_band;
+            bin2_band_list(w.bin_ws, f.N, &perm, &n_band);
+            m_dev = n_band + 1;
+        }
+    }
+    if (te && (rc = te->record(3, sr)) != BSPLAT_OK) return rc;
+    return rasterize_launch(f.N, f.channels, means2d, conics, f.colors, f.opacities, f.background, tile_ranges,
+                            f.fast_raster ? w.tile_order : nullptr, w.sorted_ids, f.W, f.H, f.tile_size, f.row0,
+                            f.row1, f.raster_mode, f.image, nullptr, m_dev, w.raster_rec, sr, peers, nullptr, nullptr,
+                            rec_ready, w.long_surv, w.long_cnt,
+                            bin2_spare_counter(w.bin_ws, f.N, M, (int64_t)f.tiles_w * f.tiles_h));
 }
 
 }  // namespace
@@ -254,9 +302,7 @@ int frame_front(int64_t N, const float* means3d, const float* log_scales, const 
 extern "C" size_t bsplat_render_workspace_bytes(int64_t N, int64_t M_capacity, int32_t width, int32_t height,
                                                 int32_t tile_size) {
     if (N < 0 || M_capacity < 0 || width <= 0 || height <= 0 || tile_size <= 0) return 0;
-    const size_t a = carve_render(nullptr, N, M_capacity, width, height, tile_size, false).total;
-    const size_t b = carve_render(nullptr, N, M_capacity, width, height, tile_size, true).total;
-    return a > b ? a : b;
+    return carve_render(nullptr, N, M_capacity, width, height, tile_size).total;
 }
 
 extern "C" int bsplat_render_fwd(int64_t N, const float* means3d, const float* log_scales, const float* quats,
@@ -266,21 +312,19 @@ extern "C" int bsplat_render_fwd(int64_t N, const float* means3d, const float* l
                                  size_t workspace_bytes, size_t* needed_bytes, bsplat_render_aux* aux,
                                  void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!cam || !image || !background || N < 0 || channels <= 0 || tile_size <= 0 || tile_size > 32)
-        return BSPLAT_E_ARG;
+    Frame f;
+    int rc = make_frame(N, means3d, log_scales, quats, opacities, colors, channels, cam, background, tile_size,
+                        semantics, flags, image, &f);
+    if (rc != BSPLAT_OK) return rc;
+    if (!image || !background || channels <= 0) return BSPLAT_E_ARG;
     if (N > 0 && (!means3d || !log_scales || !quats || !opacities || !colors)) return BSPLAT_E_ARG;
-    if (semantics != BSPLAT_SEM_TORCH && semantics != BSPLAT_SEM_GSPLAT) return BSPLAT_E_ARG;
-    const int W = cam->width, H = cam->height;
-    if (W <= 0 || H <= 0) return BSPLAT_E_ARG;
-    const int raster_mode = flags & 0xff;
-    const bool single_level = (flags & BSPLAT_FLAG_BIN_SINGLE_LEVEL) != 0;
-    const size_t image_bytes = (size_t)W * H * channels * sizeof(float);
+    const size_t image_bytes = (size_t)f.W * f.H * channels * sizeof(float);
     if (aux) { aux->n_isect = 0; aux->n_launches = 0; aux->sort_passes = 0; aux->key_bits = 0; }
 
     // fixed (N-dependent) part must fit before anything runs
-    RenderWs w = carve_render(workspace, N, 0, W, H, tile_size, single_level);
+    RenderWs w = carve_render(workspace, N, 0, f.W, f.H, tile_size);
     if (!workspace || workspace_bytes < w.total) {
-        if (needed_bytes) *needed_bytes = bsplat_render_workspace_bytes(N, 4 * N + 1024, W, H, tile_size);
+        if (needed_bytes) *needed_bytes = bsplat_render_workspace_bytes(N, 4 * N + 1024, f.W, f.H, tile_size);
         return BSPLAT_E_WORKSPACE;
     }
     if (N == 0) {
@@ -289,123 +333,58 @@ extern "C" int bsplat_render_fwd(int64_t N, const float* means3d, const float* l
     }
     StageEvents te;
     if (aux && aux->timing) {
-        int rc0 = te.create();
-        if (rc0 != BSPLAT_OK) return rc0;
+        rc = te.create();
+        if (rc != BSPLAT_OK) return rc;
     }
-    int rc = te.record(0, stream);
+    rc = te.record(0, stream);
     if (rc != BSPLAT_OK) return rc;
-    const bool fast_raster = fast_raster_for(raster_mode, tile_size, channels);
     const bool want_aux = aux && (aux->means2d || aux->conics || aux->depths || aux->radii);
     // the reference's four projection outputs are only stored when somebody reads them
-    const bool stage_outputs = single_level || !fast_raster || want_aux;
+    const bool stage_outputs = !f.fast_raster || want_aux;
     float* d_means2d = (aux && aux->means2d) ? aux->means2d : w.means2d;
     float* d_conics = (aux && aux->conics) ? aux->conics : w.conics;
     float* d_depths = (aux && aux->depths) ? aux->depths : w.depths;
     int32_t* d_radii = (aux && aux->radii) ? aux->radii : w.radii;
     int32_t* d_ranges = (aux && aux->tile_ranges) ? aux->tile_ranges : w.tile_ranges;
-
-    const int tiles_w = (W + tile_size - 1) / tile_size, tiles_h = (H + tile_size - 1) / tile_size;
-    bsplat_bin_info* d_info;
-    Bin1Ws b1 = carve_bin1(w.bin_ws, N, 0);
-    bool rec_ready = false;
-    if (single_level) {
-        rc = project_fwd_launch(N, means3d, log_scales, quats, opacities, *cam, 0.3f, semantics, d_means2d, d_conics,
-                                d_depths, d_radii, stream, nullptr, nullptr, proj_variant_of(flags));
-        if (rc != BSPLAT_OK) return rc;
-        rc = te.record(1, stream);
-        if (rc != BSPLAT_OK) return rc;
-        rc = bsplat_bin_count_scan(N, d_means2d, d_radii, 0, d_depths, W, H, tile_size, 0, tiles_h, semantics,
-                                   b1.offsets, b1.info, b1.scan_ws, b1.scan_bytes, stream);
-        d_info = b1.info;
-    } else {
-        d_info = bin2_info_ptr(w.bin_ws, N);
-        rec_ready = fast_raster;
-        rc = frame_front(N, means3d, log_scales, quats, opacities, colors, *cam, nullptr, tile_size, semantics, flags,
-                         0, tiles_h, fast_raster, stage_outputs ? d_means2d : nullptr,
-                         stage_outputs ? d_conics : nullptr, stage_outputs ? d_depths : nullptr,
-                         stage_outputs ? d_radii : nullptr, w, stream, te.on ? te.ev[1] : nullptr);
-    }
+    rc = frame_front(f, nullptr, f.fast_raster, stage_outputs ? d_means2d : nullptr, stage_outputs ? d_conics : nullptr,
+                     stage_outputs ? d_depths : nullptr, stage_outputs ? d_radii : nullptr, w, stream,
+                     te.on ? te.ev[1] : nullptr);
     if (rc != BSPLAT_OK) return rc;
     bsplat_bin_info info;
-    BSPLAT_CUDA_TRY(cudaMemcpyAsync(&info, d_info, sizeof(info), cudaMemcpyDeviceToHost, stream));
+    BSPLAT_CUDA_TRY(cudaMemcpyAsync(&info, bin2_info_ptr(w.bin_ws, N), sizeof(info), cudaMemcpyDeviceToHost, stream));
     BSPLAT_CUDA_TRY(cudaStreamSynchronize(stream));  // the single read-back of the frame (M, key range)
     const int64_t M = (int64_t)info.n_isect;
-    if (aux) { aux->n_isect = M; aux->n_launches = single_level ? 3 : 6; }
+    if (aux) { aux->n_isect = M; aux->n_launches = 6; }  // so far: project, 4 depth passes, count + scan
     if (M >= (1ll << 30)) return BSPLAT_E_OVERFLOW;
     if (M == 0) {
         // render.py:73-76: no overlaps => black image (not the background)
         BSPLAT_CUDA_TRY(cudaMemsetAsync(image, 0, image_bytes, stream));
-        BSPLAT_CUDA_TRY(cudaMemsetAsync(d_ranges, 0, (size_t)tiles_w * tiles_h * 2 * sizeof(int32_t), stream));
+        BSPLAT_CUDA_TRY(cudaMemsetAsync(d_ranges, 0, (size_t)f.tiles_w * f.tiles_h * 2 * sizeof(int32_t), stream));
         return BSPLAT_OK;
     }
-    w = carve_render(workspace, N, M, W, H, tile_size, single_level);
+    w = carve_render(workspace, N, M, f.W, f.H, tile_size);
     if (workspace_bytes < w.total) {
-        if (needed_bytes) *needed_bytes = bsplat_render_workspace_bytes(N, M + M / 4, W, H, tile_size);
+        if (needed_bytes) *needed_bytes = bsplat_render_workspace_bytes(N, M + M / 4, f.W, f.H, tile_size);
         return BSPLAT_E_WORKSPACE;
     }
-    const int32_t* sorted_ids = nullptr;
-    bool have_order = false;
-    if (single_level) {
-        b1 = carve_bin1(w.bin_ws, N, M);
-        const bsplat_key_layout layout = bsplat_make_key_layout(&info, W, H, tile_size);
-        rc = bsplat_bin_emit(N, d_means2d, d_radii, 0, d_depths, W, H, tile_size, 0, tiles_h, semantics,
-                             b1.offsets, layout, b1.keys, b1.ids, stream);
-        if (rc != BSPLAT_OK) return rc;
-        rc = te.record(2, stream);
-        if (rc != BSPLAT_OK) return rc;
-        int in_alt = 0;
-        rc = bsplat_radix_sort_pairs(M, b1.keys, b1.keys_alt, b1.ids, b1.ids_alt, 0,
-                                     layout.depth_bits + layout.tile_bits, b1.sort_ws, b1.sort_bytes, &in_alt, stream);
-        if (rc != BSPLAT_OK) return rc;
-        sorted_ids = in_alt ? b1.ids_alt : b1.ids;
-        rc = bsplat_tile_ranges(M, in_alt ? b1.keys_alt : b1.keys, layout.depth_bits, tiles_w * tiles_h, d_ranges,
-                                stream);
-        if (rc != BSPLAT_OK) return rc;
-        if (aux) {
-            aux->key_bits = layout.depth_bits + layout.tile_bits;
-            aux->sort_passes = (aux->key_bits + 7) / 8;
-            aux->n_launches = 3 + 1 + 2 + aux->sort_passes + 1 + 1;
-        }
-    } else {
-        // stage_ms: [0] projection (+ epilogue), [1] depth sort + count/scan (+ the M read-back), [2] emit + tile sort +
-        // ranges, [3] rasterizer (+ long-list pre-pass)
-        rc = te.record(2, stream);
-        if (rc != BSPLAT_OK) return rc;
-        BinParams p;
-        rc = make_bin_params(W, H, tile_size, 0, tiles_h, semantics, &p);
-        if (rc != BSPLAT_OK) return rc;
-        rc = bin2_finish(N, M, false, p, w.bin_ws, w.bin_bytes, w.sorted_ids, d_ranges, w.tile_order, stream,
-                         (flags & BSPLAT_FLAG_PACKED) != 0);
-        if (rc != BSPLAT_OK) return rc;
-        sorted_ids = w.sorted_ids;
-        have_order = true;
-        if (aux) {
-            int tb = 1;
-            while ((1 << tb) < tiles_w * tiles_h) ++tb;
-            const int tile_passes = (tb + 7) / 8;
-            aux->key_bits = 32 + tb;
-            aux->sort_passes = 4 + tile_passes;  // 4 over N items, the rest over M items
-            // project (+ epilogue), [compact,] 4 passes, count_scan | emit, tile passes, tile_finish
-            aux->n_launches = 1 + ((flags & BSPLAT_FLAG_PACKED) ? 1 : 0) + 4 + 1 + 1 + tile_passes + 1;
-        }
+    if (aux) {
+        int tb = 1;
+        while ((1 << tb) < f.tiles_w * f.tiles_h) ++tb;
+        const int tile_passes = (tb + 7) / 8;
+        aux->key_bits = 32 + tb;
+        aux->sort_passes = 4 + tile_passes;  // 4 over N items, the rest over M items
+        // project (+ epilogue), [compact,] 4 passes, count_scan | emit, tile passes, tile_finish | [long-list
+        // pre-pass,] rasterizer
+        aux->n_launches = 1 + ((flags & BSPLAT_FLAG_PACKED) ? 1 : 0) + 4 + 1 + 1 + tile_passes + 1 +
+                          (f.fast_raster ? 1 : 0) + 1;
     }
-    if (fast_raster && !have_order) {
-        rc = tile_order_launch(0, tiles_w * tiles_h, d_ranges, w.tile_order, stream);
-        if (rc != BSPLAT_OK) return rc;
-        if (aux) aux->n_launches += 1;
-    }
-    if (aux && fast_raster) aux->n_launches += rec_ready ? 1 : 2;  // [record kernel,] long-list pre-pass
-    if (aux) aux->n_launches += 1;                                   // rasterizer
-    rc = te.record(3, stream);
-    if (rc != BSPLAT_OK) return rc;
-    rc = rasterize_launch(N, channels, d_means2d, d_conics, colors, opacities, background, d_ranges,
-                          fast_raster ? w.tile_order : nullptr, sorted_ids, W, H, tile_size, 0, tiles_h, raster_mode,
-                          image, nullptr, nullptr, w.raster_rec, stream, nullptr, nullptr, nullptr, rec_ready,
-                          w.long_surv, w.long_cnt,
-                          single_level ? nullptr : bin2_spare_counter(w.bin_ws, N, M, (int64_t)tiles_w * tiles_h));
+    // stage_ms: [0] projection (+ epilogue), [1] depth sort + count/scan (+ the M read-back), [2] emit + tile sort +
+    // ranges, [3] rasterizer (+ long-list pre-pass)
+    rc = frame_back(f, w, M, /*device_m=*/false, d_means2d, d_conics, d_ranges, /*rec_ready=*/f.fast_raster, nullptr,
+                    stream, stream, nullptr, nullptr, &te);
     if (rc != BSPLAT_OK) return rc;
     if (aux && aux->sorted_ids && aux->sorted_ids_capacity >= M)
-        BSPLAT_CUDA_TRY(cudaMemcpyAsync(aux->sorted_ids, sorted_ids, (size_t)M * sizeof(int32_t),
+        BSPLAT_CUDA_TRY(cudaMemcpyAsync(aux->sorted_ids, w.sorted_ids, (size_t)M * sizeof(int32_t),
                                         cudaMemcpyDeviceToDevice, stream));
     if (te.on) {
         rc = te.record(4, stream);
@@ -426,20 +405,18 @@ extern "C" int bsplat_render_begin(int64_t N, const float* means3d, const float*
                                    int32_t semantics, void* workspace, size_t workspace_bytes,
                                    bsplat_bin_info* info_host_pinned, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!cam || !info_host_pinned || N <= 0 || tile_size <= 0 || tile_size > 32) return BSPLAT_E_ARG;
-    if (!means3d || !log_scales || !quats) return BSPLAT_E_ARG;
-    if (semantics != BSPLAT_SEM_TORCH && semantics != BSPLAT_SEM_GSPLAT) return BSPLAT_E_ARG;
-    const int W = cam->width, H = cam->height;
-    if (W <= 0 || H <= 0) return BSPLAT_E_ARG;
-    RenderWs w = carve_render(workspace, N, 0, W, H, tile_size, false);
-    if (!workspace || workspace_bytes < w.total) return BSPLAT_E_WORKSPACE;
-    const int tiles_h = (H + tile_size - 1) / tile_size;
-    // (colours arrive with bsplat_render_end: the raster records are built there, from the stage outputs kept here)
-    int rc = frame_front(N, means3d, log_scales, quats, opacities, nullptr, *cam, nullptr, tile_size, semantics, 0, 0,
-                         tiles_h, false, w.means2d, w.conics, w.depths, w.radii, w, stream);
+    Frame f;
+    int rc = make_frame(N, means3d, log_scales, quats, opacities, nullptr, 0, cam, nullptr, tile_size, semantics, 0,
+                        nullptr, &f);
     if (rc != BSPLAT_OK) return rc;
-    bsplat_bin_info* d_info = bin2_info_ptr(w.bin_ws, N);
-    BSPLAT_CUDA_TRY(cudaMemcpyAsync(info_host_pinned, d_info, sizeof(bsplat_bin_info), cudaMemcpyDeviceToHost, stream));
+    if (!info_host_pinned || N <= 0 || !means3d || !log_scales || !quats) return BSPLAT_E_ARG;
+    RenderWs w = carve_render(workspace, N, 0, f.W, f.H, tile_size);
+    if (!workspace || workspace_bytes < w.total) return BSPLAT_E_WORKSPACE;
+    // (colours arrive with bsplat_render_end: the raster records are built there, from the stage outputs kept here)
+    rc = frame_front(f, nullptr, false, w.means2d, w.conics, w.depths, w.radii, w, stream);
+    if (rc != BSPLAT_OK) return rc;
+    BSPLAT_CUDA_TRY(cudaMemcpyAsync(info_host_pinned, bin2_info_ptr(w.bin_ws, N), sizeof(bsplat_bin_info),
+                                    cudaMemcpyDeviceToHost, stream));
     return BSPLAT_OK;
 }
 
@@ -448,35 +425,24 @@ extern "C" int bsplat_render_end(int64_t N, int64_t M, const float* colors, cons
                                  int32_t semantics, int32_t flags, float* image, void* workspace,
                                  size_t workspace_bytes, size_t* needed_bytes, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!cam || !image || !background || N <= 0 || M < 0 || channels <= 0) return BSPLAT_E_ARG;
-    if (tile_size <= 0 || tile_size > 32) return BSPLAT_E_ARG;
-    if (!colors || !opacities) return BSPLAT_E_ARG;
-    if (semantics != BSPLAT_SEM_TORCH && semantics != BSPLAT_SEM_GSPLAT) return BSPLAT_E_ARG;
+    // bsplat_render_begin ran without BSPLAT_FLAG_PACKED: only the rasterizer mode of `flags` applies here
+    Frame f;
+    int rc = make_frame(N, nullptr, nullptr, nullptr, opacities, colors, channels, cam, background, tile_size,
+                        semantics, flags & 0xff, image, &f);
+    if (rc != BSPLAT_OK) return rc;
+    if (!image || !background || channels <= 0 || N <= 0 || M < 0 || !colors || !opacities) return BSPLAT_E_ARG;
     if (M >= (1ll << 30)) return BSPLAT_E_OVERFLOW;
-    const int W = cam->width, H = cam->height;
-    if (W <= 0 || H <= 0) return BSPLAT_E_ARG;
-    const int raster_mode = flags & 0xff;
-    const int tiles_h = (H + tile_size - 1) / tile_size;
     if (M == 0) {
-        BSPLAT_CUDA_TRY(cudaMemsetAsync(image, 0, (size_t)W * H * channels * sizeof(float), stream));
+        BSPLAT_CUDA_TRY(cudaMemsetAsync(image, 0, (size_t)f.W * f.H * channels * sizeof(float), stream));
         return BSPLAT_OK;
     }
-    RenderWs w = carve_render(workspace, N, M, W, H, tile_size, false);
+    RenderWs w = carve_render(workspace, N, M, f.W, f.H, tile_size);
     if (!workspace || workspace_bytes < w.total) {
         if (needed_bytes) *needed_bytes = w.total;
         return BSPLAT_E_WORKSPACE;
     }
-    BinParams p;
-    int rc = make_bin_params(W, H, tile_size, 0, tiles_h, semantics, &p);
-    if (rc != BSPLAT_OK) return rc;
-    rc = bin2_finish(N, M, false, p, w.bin_ws, w.bin_bytes, w.sorted_ids, w.tile_ranges, w.tile_order, stream, false);
-    if (rc != BSPLAT_OK) return rc;
-    const bool fast_raster = fast_raster_for(raster_mode, tile_size, channels);
-    return rasterize_launch(N, channels, w.means2d, w.conics, colors, opacities, background, w.tile_ranges,
-                            fast_raster ? w.tile_order : nullptr, w.sorted_ids, W, H, tile_size, 0, tiles_h,
-                            raster_mode, image, nullptr, nullptr, w.raster_rec, stream, nullptr, nullptr, nullptr,
-                            /*rec_ready=*/false, w.long_surv, w.long_cnt,
-                            bin2_spare_counter(w.bin_ws, N, M, (int64_t)p.tiles_w * p.tiles_h));
+    return frame_back(f, w, M, /*device_m=*/false, w.means2d, w.conics, w.tile_ranges, /*rec_ready=*/false, nullptr,
+                      stream, stream, nullptr, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -539,27 +505,24 @@ extern "C" int bsplat_render_enqueue_band_p2p(int64_t N, const float* means3d, c
     }
     cudaStream_t sb = (cudaStream_t)stream_bin_;
     cudaStream_t sr = stream_raster_ ? (cudaStream_t)stream_raster_ : sb;
-    if (!cam || !image || !background || N <= 0 || M_capacity <= 0 || channels <= 0 || tile_size <= 0 ||
-        tile_size > 32)
-        return BSPLAT_E_ARG;
+    Frame f;
+    int rc = make_frame(N, means3d, log_scales, quats, opacities, colors, channels, cam, background, tile_size,
+                        semantics, flags, image, &f);
+    if (rc != BSPLAT_OK) return rc;
+    if (!image || !background || channels <= 0 || N <= 0 || M_capacity <= 0) return BSPLAT_E_ARG;
     if (!means3d || !log_scales || !quats || !opacities || !colors) return BSPLAT_E_ARG;
-    if (semantics != BSPLAT_SEM_TORCH && semantics != BSPLAT_SEM_GSPLAT) return BSPLAT_E_ARG;
     if (M_capacity >= (1ll << 30)) return BSPLAT_E_OVERFLOW;
     if (sr != sb && !event_bin_done) return BSPLAT_E_ARG;
-    const int W = cam->width, H = cam->height;
-    if (W <= 0 || H <= 0) return BSPLAT_E_ARG;
-    const int raster_mode = flags & 0xff;
-    RenderWs w = carve_render(workspace, N, M_capacity, W, H, tile_size, false);
+    RenderWs w = carve_render(workspace, N, M_capacity, f.W, f.H, tile_size);
     if (!workspace || workspace_bytes < w.total) {
         if (needed_bytes) *needed_bytes = w.total;
         return BSPLAT_E_WORKSPACE;
     }
-    const int tiles_h = (H + tile_size - 1) / tile_size;
-    const int row0 = tile_row_begin < 0 ? 0 : tile_row_begin;
-    const int row1 = tile_row_end > tiles_h ? tiles_h : tile_row_end;
-    bsplat_bin_info* d_info = bin2_info_ptr(w.bin_ws, N);
-    if (row1 <= row0) {
+    f.row0 = tile_row_begin < 0 ? 0 : tile_row_begin;
+    f.row1 = tile_row_end > f.tiles_h ? f.tiles_h : tile_row_end;
+    if (f.row1 <= f.row0) {
         // empty band: nothing to write, but the caller's status protocol still holds -- a zeroed info and the event
+        bsplat_bin_info* d_info = bin2_info_ptr(w.bin_ws, N);
         BSPLAT_CUDA_TRY(cudaMemsetAsync(d_info, 0, sizeof(bsplat_bin_info), sb));
         if (info_host_pinned)
             BSPLAT_CUDA_TRY(cudaMemcpyAsync(info_host_pinned, d_info, sizeof(bsplat_bin_info), cudaMemcpyDeviceToHost, sb));
@@ -575,51 +538,15 @@ extern "C" int bsplat_render_enqueue_band_p2p(int64_t N, const float* means3d, c
         BSPLAT_CUDA_TRY(cudaMemcpyAsync(w.cam_dev, cam, sizeof(bsplat_camera), cudaMemcpyDefault, sb));
         cam_dev = w.cam_dev;
     }
-    const bool fast_raster = fast_raster_for(raster_mode, tile_size, channels);
     const PdlScope pdl_scope(sr == sb);  // two streams = overlapped pipeline: plain launches (common.cuh)
     // the faithful rasterizer reads the stage outputs; the fast one only needs the records of the projection epilogue
-    int rc = frame_front(N, means3d, log_scales, quats, opacities, colors, *cam, cam_dev, tile_size, semantics, flags,
-                         row0, row1, fast_raster, fast_raster ? nullptr : w.means2d, fast_raster ? nullptr : w.conics,
-                         fast_raster ? nullptr : w.depths, fast_raster ? nullptr : w.radii, w, sb);
+    const bool stage_outputs = !f.fast_raster;
+    rc = frame_front(f, cam_dev, f.fast_raster, stage_outputs ? w.means2d : nullptr, stage_outputs ? w.conics : nullptr,
+                     stage_outputs ? w.depths : nullptr, stage_outputs ? w.radii : nullptr, w, sb);
     if (rc != BSPLAT_OK) return rc;
-    BinParams p;
-    rc = make_bin_params(W, H, tile_size, row0, row1, semantics, &p);
-    if (rc != BSPLAT_OK) return rc;
-    // the bin info reaches the host as a store from the last binning kernel when the block is device-accessible
-    // (pinned memory under UVA); a copy-engine transfer would queue behind image downloads of earlier frames
-    bool info_direct = false;
-    if (info_host_pinned) {
-        cudaPointerAttributes attr;
-        if (cudaPointerGetAttributes(&attr, info_host_pinned) == cudaSuccess && attr.type == cudaMemoryTypeHost &&
-            attr.devicePointer == (void*)info_host_pinned)
-            info_direct = true;
-        else
-            (void)cudaGetLastError();
-    }
-    rc = bin2_finish(N, M_capacity, /*device_m=*/true, p, w.bin_ws, w.bin_bytes, w.sorted_ids, w.tile_ranges,
-                     w.tile_order, sb, (flags & BSPLAT_FLAG_PACKED) != 0, info_direct ? info_host_pinned : nullptr);
-    if (rc != BSPLAT_OK) return rc;
-    if (info_host_pinned && !info_direct)
-        BSPLAT_CUDA_TRY(cudaMemcpyAsync(info_host_pinned, d_info, sizeof(bsplat_bin_info), cudaMemcpyDeviceToHost, sb));
-    if (sr != sb) {
-        BSPLAT_CUDA_TRY(cudaEventRecord((cudaEvent_t)event_bin_done, sb));
-        BSPLAT_CUDA_TRY(cudaStreamWaitEvent(sr, (cudaEvent_t)event_bin_done, 0));
-    }
-    // "no intersections at all => all-zero image" (render.py:73-76) is a whole-frame rule: a partial band decides it
-    // from the number of Gaussians that own a tile anywhere in the frame (counted by the compaction pass)
-    const bool band_partial = row0 > 0 || row1 < tiles_h;
-    const unsigned long long* m_dev = reinterpret_cast<const unsigned long long*>(d_info);
-    if (band_partial) {
-        const int32_t* perm;
-        const unsigned long long* n_band;
-        bin2_band_list(w.bin_ws, N, &perm, &n_band);
-        m_dev = n_band + 1;
-    }
-    return rasterize_launch(N, channels, w.means2d, w.conics, colors, opacities, background, w.tile_ranges,
-                            fast_raster ? w.tile_order : nullptr, w.sorted_ids, W, H, tile_size, row0, row1,
-                            raster_mode, image, nullptr, m_dev, w.raster_rec, sr, &peers, nullptr, nullptr,
-                            /*rec_ready=*/fast_raster, w.long_surv, w.long_cnt,
-                            bin2_spare_counter(w.bin_ws, N, M_capacity, (int64_t)p.tiles_w * p.tiles_h));
+    return frame_back(f, w, M_capacity, /*device_m=*/true, w.means2d, w.conics, w.tile_ranges,
+                      /*rec_ready=*/f.fast_raster, &peers, sb, sr, (cudaEvent_t)event_bin_done, info_host_pinned,
+                      nullptr);
 }
 
 extern "C" size_t bsplat_render_host_scratch_bytes(int64_t N, int32_t channels, int32_t width, int32_t height) {

@@ -23,7 +23,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .binning import bin_gaussians_to_tiles_cuda
+from .binning import bin_gaussians_to_tiles_cuda, read_bin_info
 from .projection import project_gaussians_cuda
 from .rasterization import rasterize_gaussians_cuda
 from .render import TILE_SIZE, render_fused
@@ -375,7 +375,7 @@ class RowBandRenderer:
 
     def check(self) -> int:
         torch.cuda.synchronize(self.dev)
-        info = _lib.BsplatBinInfo.from_buffer_copy(self.info.numpy().tobytes())
+        info = read_bin_info(self.info)
         if info.reserved[1]:
             need = int(info.n_isect)
             self._resize(int(1.25 * need) + 65536)  # the next render() fits; this frame must be redone

@@ -17,8 +17,17 @@ from typing import Sequence
 import torch
 
 from . import _lib
+from .binning import read_bin_info
 from .rasterization import RASTER_MODES
 from .utils import Camera
+
+
+def _gaussians(t, N: int, C: int) -> list:
+    """The five Gaussian arrays (means3d, scales, quats, opacities, features) as contiguous float32, opacities flat."""
+    q = [_lib.as_f32(t[0], "means3d"), _lib.as_f32(t[1], "scales"), _lib.as_f32(t[2], "quats"),
+         _lib.as_f32(t[3], "opacities").reshape(-1), _lib.as_f32(t[4], "features")]
+    assert q[0].shape[0] == N and q[4].shape == (N, C)
+    return q
 
 
 class FramePipeline:
@@ -53,7 +62,7 @@ class FramePipeline:
 
     def _end(self, slot: int, g, cam_struct, background, image) -> int:
         self.events[slot].synchronize()  # host waits for begin(k) only; the other stream keeps the GPU busy
-        M = int(_lib.BsplatBinInfo.from_buffer_copy(self.info[slot].numpy().tobytes()).n_isect)
+        M = int(read_bin_info(self.info[slot]).n_isect)
         s = self.streams[slot]
         needed = c_size_t(0)
         for attempt in range(2):
@@ -84,15 +93,10 @@ class FramePipeline:
         ``scene_of`` (optional): callable k -> (means3d, scales, quats, opacities, features) giving frame k
         its own Gaussian set of the same N (dynamic scenes; bench.py rotates copies so that the inputs
         touched between two uses of one copy exceed the L2)."""
-        def prep(t):
-            q = [_lib.as_f32(t[0], "means3d"), _lib.as_f32(t[1], "scales"), _lib.as_f32(t[2], "quats"),
-                 _lib.as_f32(t[3], "opacities").reshape(-1), _lib.as_f32(t[4], "features")]
-            assert q[0].shape[0] == self.N and q[4].shape == (self.N, self.C)
-            return q
-        g0 = prep((means3d, scales, quats, opacities, features))
-        gs = [g0] * len(cameras) if scene_of is None else [prep(scene_of(k)) for k in range(len(cameras))]
-        bg = _lib.as_f32(background, "background").to(self.dev)
+        g0 = _gaussians((means3d, scales, quats, opacities, features), self.N, self.C)
         n = len(cameras)
+        gs = [g0] * n if scene_of is None else [_gaussians(scene_of(k), self.N, self.C) for k in range(n)]
+        bg = _lib.as_f32(background, "background").to(self.dev)
         if out is None:
             out = torch.empty((n, self.H, self.W, self.C), dtype=torch.float32, device=self.dev)
         cams = [_lib.camera_struct(c) for c in cameras]
@@ -167,14 +171,9 @@ class OverlappedPipeline:
     def render(self, means3d, scales, quats, opacities, features, cameras: Sequence[Camera], background,
                out: torch.Tensor | None = None, scene_of=None) -> torch.Tensor:
         """Render all cameras; images [n, H, W, C] (or a ring, see FramePipeline.render)."""
-        def prep(t):
-            q = [_lib.as_f32(t[0], "means3d"), _lib.as_f32(t[1], "scales"), _lib.as_f32(t[2], "quats"),
-                 _lib.as_f32(t[3], "opacities").reshape(-1), _lib.as_f32(t[4], "features")]
-            assert q[0].shape[0] == self.N and q[4].shape == (self.N, self.C)
-            return q
-        g0 = prep((means3d, scales, quats, opacities, features))
+        g0 = _gaussians((means3d, scales, quats, opacities, features), self.N, self.C)
         n = len(cameras)
-        gs = [g0] * n if scene_of is None else [prep(scene_of(k)) for k in range(n)]
+        gs = [g0] * n if scene_of is None else [_gaussians(scene_of(k), self.N, self.C) for k in range(n)]
         bg = _lib.as_f32(background, "background").to(self.dev)
         if out is None:
             out = torch.empty((n, self.H, self.W, self.C), dtype=torch.float32, device=self.dev)
@@ -208,7 +207,7 @@ class OverlappedPipeline:
         redone = 0
         max_m = 0
         for k in range(n):
-            info = _lib.BsplatBinInfo.from_buffer_copy(infos[k].numpy().tobytes())
+            info = read_bin_info(infos[k])
             max_m = max(max_m, int(info.n_isect))
             if info.reserved[1]:
                 redone += 1
@@ -217,7 +216,7 @@ class OverlappedPipeline:
             self.m_cap = int(max_m * 1.25) + 4096
             self._alloc_all()
             for k in range(n):
-                info = _lib.BsplatBinInfo.from_buffer_copy(infos[k].numpy().tobytes())
+                info = read_bin_info(infos[k])
                 if info.reserved[1]:
                     with torch.cuda.device(self.dev):
                         self.ev_bin[0].record(self.s_bin)
@@ -243,10 +242,8 @@ class GraphRenderer:
                  raster_mode: str = "fast"):
         self.dev = means3d.device
         self.L = _lib.require_device(self.dev)
-        self.g = [_lib.as_f32(means3d, "means3d").clone(), _lib.as_f32(scales, "scales").clone(),
-                  _lib.as_f32(quats, "quats").clone(), _lib.as_f32(opacities, "opacities").reshape(-1).clone(),
-                  _lib.as_f32(features, "features").clone()]
-        self.N, self.C = self.g[4].shape
+        self.N, self.C = features.shape
+        self.g = [t.clone() for t in _gaussians((means3d, scales, quats, opacities, features), self.N, self.C)]
         self.W, self.H, self.ts = int(camera.W), int(camera.H), int(tile_size)
         self.bg = _lib.as_f32(background, "background").to(self.dev).clone()
         self.image = torch.empty((self.H, self.W, self.C), dtype=torch.float32, device=self.dev)
@@ -254,7 +251,7 @@ class GraphRenderer:
         nbytes = self.L.bsplat_render_workspace_bytes(self.N, self.m_cap, self.W, self.H, self.ts)
         self.ws = torch.empty(nbytes, dtype=torch.uint8, device=self.dev)
         # pinned host blocks the graph reads / writes at replay time
-        self.cam_host = torch.zeros(ctypes_sizeof_camera(), dtype=torch.uint8).pin_memory()
+        self.cam_host = torch.zeros(ctypes.sizeof(_lib.BsplatCamera), dtype=torch.uint8).pin_memory()
         self.info_host = torch.zeros(32, dtype=torch.uint8).pin_memory()
         self._write_camera(camera)
         flags = RASTER_MODES[raster_mode] | _lib.FLAG_CAMERA_INDIRECT
@@ -282,7 +279,6 @@ class GraphRenderer:
         if int(camera.W) != self.W or int(camera.H) != self.H:
             raise ValueError("GraphRenderer: the image size is fixed at capture time")
         cs = _lib.camera_struct(camera)
-        import ctypes
         ctypes.memmove(self.cam_host.data_ptr(), ctypes.addressof(cs), ctypes.sizeof(cs))
 
     def update_gaussians(self, means3d=None, scales=None, quats=None, opacities=None, features=None) -> None:
@@ -307,16 +303,11 @@ class GraphRenderer:
     def check(self) -> int:
         """Synchronise; returns M of the last frame, raises if it exceeded the captured capacity."""
         self.stream.synchronize()
-        info = _lib.BsplatBinInfo.from_buffer_copy(self.info_host.numpy().tobytes())
+        info = read_bin_info(self.info_host)
         if info.reserved[1]:
             raise RuntimeError(f"GraphRenderer: {int(info.n_isect)} intersections exceed the captured capacity "
                                f"{self.m_cap}; rebuild with a larger m_capacity")
         return int(info.n_isect)
-
-
-def ctypes_sizeof_camera() -> int:
-    import ctypes
-    return ctypes.sizeof(_lib.BsplatCamera)
 
 
 class HostFramePipeline:
@@ -409,7 +400,7 @@ class HostFramePipeline:
             self.last_timeline = [(ev0.elapsed_time(ev_ras[k]), ev0.elapsed_time(ev_dl[k]), ev0.elapsed_time(ev_out[k]))
                                   for k in range(n)]
         for k in range(n):
-            info = _lib.BsplatBinInfo.from_buffer_copy(infos[k].numpy().tobytes())
+            info = read_bin_info(infos[k])
             if info.reserved[1]:
                 raise RuntimeError(f"frame {k}: {int(info.n_isect)} intersections exceed the pair capacity "
                                    f"{core.m_cap}; construct HostFramePipeline with a larger m_capacity")

@@ -160,12 +160,10 @@ _last_M: dict = {}
 
 
 def render_fused(means3d, scales, quats, opacities, colors, camera, background, tile_size=TILE_SIZE,
-                 semantics=_lib.SEM_TORCH, raster_mode="fast", return_aux=False, timing=False,
-                 bin_algo="two_level", packed=False, proj_fma=False, proj_fast=False):
+                 semantics=_lib.SEM_TORCH, raster_mode="fast", return_aux=False, timing=False, packed=False):
     """One C call per frame (include/bsplat.h: bsplat_render_fwd). Device tensors in, image out.
     ``packed``: gsplat's packed layout -- Gaussians that own no tile are compacted away right after projection
-    (same image and lists; only pays under the gsplat rule set, where culled Gaussians own no tile).
-    ``proj_fma``: the A/B build of the projection kernel with FMA contraction allowed."""
+    (same image and lists; only pays under the gsplat rule set, where culled Gaussians own no tile)."""
     dev = means3d.device
     L = _lib.require_device(dev)
     means3d = _lib.as_f32(means3d, "means3d"); scales = _lib.as_f32(scales, "scales")
@@ -196,9 +194,7 @@ def render_fused(means3d, scales, quats, opacities, colors, camera, background, 
             outs["sorted_ids"] = torch.empty((cap,), dtype=torch.int32, device=dev)
             aux.sorted_ids, aux.sorted_ids_capacity = outs["sorted_ids"].data_ptr(), cap
     needed = c_size_t(0)
-    flags = RASTER_MODES[raster_mode] | (_lib.FLAG_BIN_SINGLE_LEVEL if bin_algo == "single" else 0)
-    flags |= (_lib.FLAG_PACKED if packed else 0) | (_lib.FLAG_PROJ_FMA if proj_fma else 0)
-    flags |= _lib.FLAG_PROJ_FAST if proj_fast else 0
+    flags = RASTER_MODES[raster_mode] | (_lib.FLAG_PACKED if packed else 0)
     with torch.cuda.device(dev):
         for _attempt in range(3):
             rc = L.bsplat_render_fwd(N, _lib.ptr(means3d), _lib.ptr(scales), _lib.ptr(quats),

@@ -5,7 +5,7 @@ import torch
 
 import mojosplat_b200 as ms
 from helpers import audit_inputs, image_gate, scene_on
-from mojosplat_b200 import synthetic
+from mojosplat_b200 import binning, synthetic
 from oracle import oracle
 
 pytestmark = pytest.mark.gpu
@@ -20,7 +20,7 @@ def oracle_render(sc, **kw):
 
 @pytest.mark.parametrize("cfg,N", [("config1_1k_256", None), ("config2_100k_1080p", 20_000),
                                    ("config3_1m_1080p", 200_000), ("config3_1m_1080p", 1_000_000)])
-def test_render_end_to_end_vs_oracle(cuda_device, cfg, N):
+def test_render_end_to_end_vs_oracle_and_single_level(cuda_device, cfg, N):
     sc = synthetic.make_scene(cfg, N=N)
     ref = oracle_render(sc)
     (m, s, q, o, c), cam = scene_on(sc, cuda_device)
@@ -33,10 +33,11 @@ def test_render_end_to_end_vs_oracle(cuda_device, cfg, N):
     # stage outputs of the fused path: binning must be bit-exact when the projected inputs agree
     img2, aux = ms.render_fused(m, s, q, o, c, cam, sc.background.to(cuda_device), return_aux=True)
     assert torch.equal(img, img2)
-    img3, aux3 = ms.render_fused(m, s, q, o, c, cam, sc.background.to(cuda_device), return_aux=True, bin_algo="single")
-    assert torch.equal(img, img3) and torch.equal(aux["tile_ranges"], aux3["tile_ranges"])
-    if aux.get("sorted_ids") is not None and aux3.get("sorted_ids") is not None:
-        assert torch.equal(aux["sorted_ids"], aux3["sorted_ids"])
+    # the frame's two-level lists equal the stand-alone single-level binning of its own stage outputs
+    ids1, ranges1 = binning.bin_gaussians_to_tiles_cuda(aux["means2d"], aux["radii"], aux["depths"], cam.H, cam.W, 16,
+                                                        algo="single")
+    assert torch.equal(aux["tile_ranges"], ranges1)
+    assert aux["sorted_ids"] is not None and torch.equal(aux["sorted_ids"], ids1)
     assert aux["n_isect"] == ref["sorted_ids"].shape[0] or abs(aux["n_isect"] - ref["sorted_ids"].shape[0]) <= 8
     if np.array_equal(aux["radii"].cpu().numpy(), ref["radii"]) and \
             np.array_equal(aux["means2d"].cpu().numpy(), ref["means2d"]):
