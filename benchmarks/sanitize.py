@@ -1,5 +1,5 @@
 """compute-sanitizer workload: every kernel of libbsplat.so on small scenes (both rule sets, packed layout, row bands,
-long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward).  Run as
+long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward, SSIM + L1 loss).  Run as
 
     compute-sanitizer --tool memcheck  python benchmarks/sanitize.py
     compute-sanitizer --tool racecheck python benchmarks/sanitize.py
@@ -73,5 +73,8 @@ for cfg, N, sem in [("config1_1k_256", None, "cuda"), ("config3_1m_1080p", 8000 
     p3 = [x.clone().requires_grad_(True) for x in (g[0], g[1], g[2], coeffs)]
     ms.render_gaussians_diff(p3[0], p3[1], p3[2], g[3], p3[3], sc.camera, sh_degree=3, background_color=bg,
                              backend=sem).sum().backward()
+    # photometric loss: fused SSIM + L1 forward (with the gradient maps) and backward
+    li = img2.detach().clone().requires_grad_(True)
+    ms.l1_dssim_loss(li, img.detach()).backward()
     torch.cuda.synchronize()
     print(cfg, sem, "ok", float(img.mean()), flush=True)

@@ -28,6 +28,8 @@
  *                             kernels/rasterization.mojo:138-162, checked against torch autograd
  *   bsplat_project_bwd / bsplat_sh_bwd   no reference counterpart: backward of the projection and of the SH
  *                             colours (render_gaussians_diff), checked against torch autograd
+ *   bsplat_ssim_fwd / bsplat_ssim_bwd   no reference counterpart: the photometric training loss (3DGS's SSIM and
+ *                             L1 on one image pair, forward + backward), checked against torch autograd
  *   bsplat_render_fwd         mojosplat/render.py:12-103 render_gaussians (the three stages chained
  *                              on one stream with a single 16-byte read-back)
  *   bsplat_render_enqueue     same without the read-back (device-side M, two-stream overlap, graph capture)
@@ -235,6 +237,23 @@ int bsplat_sh_eval(int64_t N, int32_t degree, int32_t K_stored, const float* coe
  * where r + 0.5 >= 0. */
 int bsplat_sh_bwd(int64_t N, int32_t degree, int32_t K_stored, const float* coeffs, const float* means3d,
                   const float* campos_host, const float* v_colors, float* v_coeffs, float* v_means3d, void* stream);
+
+/* ---- photometric training loss (no reference counterpart) ---------------------------------- */
+/* SSIM as 3DGS defines it (11x11 Gaussian window, sigma 1.5, per channel, zero padding 5, C1 = 0.01^2, C2 = 0.03^2,
+ * mean over all H*W*C values) and the L1 term mean |img - target|, for fp32 images [H, W, C] with H, W >= 1 and
+ * 1 <= C <= 4 (else BSPLAT_E_ARG).  Nothing is read back to the host; both sums are deterministic (per-CTA partials
+ * in the workspace, added in a fixed order).
+ * fwd: writes out2 (device) = [mean SSIM, mean L1].  maps [3, H, W, C] (NULL when no gradient is wanted) receives the
+ * per-pixel factors the backward convolves: dS/dmu_x - 2 mu_x dS/dsigma_x^2 - mu_y dS/dsigma_xy, dS/dsigma_x^2,
+ * dS/dsigma_xy.  A workspace shorter than bsplat_ssim_workspace_bytes (8-byte aligned) is BSPLAT_E_WORKSPACE with
+ * *needed_bytes (nullable) set. */
+size_t bsplat_ssim_workspace_bytes(int32_t H, int32_t W, int32_t C);
+int bsplat_ssim_fwd(int32_t H, int32_t W, int32_t C, const float* img, const float* target, float* out2,
+                    float* maps, void* workspace, size_t workspace_bytes, size_t* needed_bytes, void* stream);
+/* bwd: v_out2 (device) = [dL/d mean SSIM, dL/d mean L1]; WRITES v_img [H, W, C] = d loss / d img (maps from
+ * bsplat_ssim_fwd on the same images; the L1 term's derivative is sign(img - target), 0 where they are equal). */
+int bsplat_ssim_bwd(int32_t H, int32_t W, int32_t C, const float* img, const float* target, const float* maps,
+                    const float* v_out2, float* v_img, void* stream);
 
 /* ---- stage 3, training side (SURVEY.md 8f rank 1; the reference is forward-only, render.py:11) --------- */
 /* Forward with the faithful arithmetic (kernels/rasterization.mojo:138-162) that also stores what the

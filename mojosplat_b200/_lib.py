@@ -42,7 +42,7 @@ SYMBOLS = [
     "bsplat_bin2_finish", "bsplat_tile_order", "bsplat_render_begin", "bsplat_render_end",
     "bsplat_render_enqueue", "bsplat_rasterize_workspace_bytes", "bsplat_rasterize_fwd_train",
     "bsplat_rasterize_fwd_train_fast", "bsplat_rasterize_bwd", "bsplat_rasterize_bwd_fast", "bsplat_render_enqueue_band", "bsplat_render_enqueue_band_p2p", "bsplat_sh_eval",
-    "bsplat_project_bwd", "bsplat_sh_bwd",
+    "bsplat_project_bwd", "bsplat_sh_bwd", "bsplat_ssim_workspace_bytes", "bsplat_ssim_fwd", "bsplat_ssim_bwd",
 ]
 
 
@@ -168,6 +168,14 @@ def load() -> ctypes.CDLL:
                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
         L.bsplat_sh_bwd.argtypes = [c_int64, c_int32, c_int32, c_void_p, c_void_p, POINTER(c_float * 3), c_void_p,
                                     c_void_p, c_void_p, c_void_p]
+        L.bsplat_ssim_workspace_bytes.restype = c_size_t
+        L.bsplat_ssim_workspace_bytes.argtypes = [c_int32, c_int32, c_int32]
+        L.bsplat_ssim_fwd.restype = ctypes.c_int
+        L.bsplat_ssim_fwd.argtypes = [c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_size_t, POINTER(c_size_t), c_void_p]
+        L.bsplat_ssim_bwd.restype = ctypes.c_int
+        L.bsplat_ssim_bwd.argtypes = [c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_void_p]
         L.bsplat_rasterize_stats.argtypes = [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                              c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
                                              c_int32, c_void_p, c_void_p, c_void_p]
