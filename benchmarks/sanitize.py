@@ -1,5 +1,5 @@
 """compute-sanitizer workload: every kernel of libbsplat.so on small scenes (both rule sets, packed layout, row bands,
-long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward, SSIM + L1 loss).  Run as
+long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward, SSIM + L1 loss, densification).  Run as
 
     compute-sanitizer --tool memcheck  python benchmarks/sanitize.py
     compute-sanitizer --tool racecheck python benchmarks/sanitize.py
@@ -76,5 +76,16 @@ for cfg, N, sem in [("config1_1k_256", None, "cuda"), ("config3_1m_1080p", 8000 
     # photometric loss: fused SSIM + L1 forward (with the gradient maps) and backward
     li = img2.detach().clone().requires_grad_(True)
     ms.l1_dssim_loss(li, img.detach()).backward()
+    # adaptive density control: statistics, plan and one apply over every tensor role (clones, splits and prunes)
+    st = ms.DensifyStats(sc.N, dev)
+    st.accumulate(torch.randn(sc.N, 2, device=dev) * 1e-3, aux["radii"], sc.camera.W, sc.camera.H)
+    dp = dict(means3d=g[0], scales=g[1], quats=g[2], opacities=g[3], colors=g[4], sh=coeffs)
+    dp = {k: v.clone().requires_grad_(True) for k, v in dp.items()}
+    dopt = torch.optim.Adam(list(dp.values()))
+    for v in dp.values():
+        v.grad = torch.ones_like(v)
+    dopt.step()
+    dnew, dcounts = ms.densify_and_prune(dp, st, 1.0, min_opacity=0.3, optimizer=dopt)
+    assert dcounts["n_out"] == dnew["sh"].shape[0] > 0
     torch.cuda.synchronize()
     print(cfg, sem, "ok", float(img.mean()), flush=True)

@@ -30,6 +30,8 @@
  *                             colours (render_gaussians_diff), checked against torch autograd
  *   bsplat_ssim_fwd / bsplat_ssim_bwd   no reference counterpart: the photometric training loss (3DGS's SSIM and
  *                             L1 on one image pair, forward + backward), checked against torch autograd
+ *   bsplat_densify_stats / _plan / _apply   no reference counterpart: adaptive density control (3DGS's gradient
+ *                             statistics and densify_and_prune), checked against a torch restatement
  *   bsplat_render_fwd         mojosplat/render.py:12-103 render_gaussians (the three stages chained
  *                              on one stream with a single 16-byte read-back)
  *   bsplat_render_enqueue     same without the read-back (device-side M, two-stream overlap, graph capture)
@@ -254,6 +256,56 @@ int bsplat_ssim_fwd(int32_t H, int32_t W, int32_t C, const float* img, const flo
  * bsplat_ssim_fwd on the same images; the L1 term's derivative is sign(img - target), 0 where they are equal). */
 int bsplat_ssim_bwd(int32_t H, int32_t W, int32_t C, const float* img, const float* target, const float* maps,
                     const float* v_out2, float* v_img, void* stream);
+
+/* ---- adaptive density control (no reference counterpart) ----------------------------------- */
+/* 3DGS's densify_and_prune.  Thresholds are fp32 values the caller computes in double and rounds once; every
+ * decision compares in log space (no exp).  +inf / INT32_MAX (and -inf for min_opacity) disable a prune rule. */
+typedef struct bsplat_densify_params {
+    float grad_threshold;       /* clone / split when count > 0 and grad2d / count >= this */
+    float log_clone_max_scale;  /* log(percent_dense * scene_extent): max log-scale <= this clones, else splits */
+    float min_opacity;          /* prune when opacity < this */
+    float log_max_world_scale;  /* prune when the row's max log-scale > this (split children: their reduced scale) */
+    int32_t max_screen_radius;  /* prune when max_radius > this */
+    int32_t reserved;
+} bsplat_densify_params;
+/* roles of a bsplat_densify_tensor */
+#define BSPLAT_DENSIFY_COPY 0        /* every output row copies its parent's row */
+#define BSPLAT_DENSIFY_MEANS 1       /* [N, 3] means3d: split children mu + R(q / |q|) (exp(s) * noise[k, c]) */
+#define BSPLAT_DENSIFY_LOG_SCALES 2  /* [N, 3] log-scales: split children s - (float)ln 1.6 */
+#define BSPLAT_DENSIFY_STATE 3       /* optimizer state: kept rows keep theirs, clone copies and split children get 0 */
+typedef struct bsplat_densify_tensor {
+    const float* src;  /* [N, width] */
+    float* dst;        /* [n_out, width], not src */
+    int32_t width;     /* 1..256 floats per row */
+    int32_t role;
+} bsplat_densify_tensor;
+typedef struct bsplat_densify_counts {
+    int64_t n_out;     /* output rows: N + n_clone + n_split - n_pruned */
+    int64_t n_clone;   /* clone decisions */
+    int64_t n_split;   /* split decisions (rows of the noise tensor), pruned ones included */
+    int64_t n_pruned;  /* output rows dropped by the prune rules */
+} bsplat_densify_counts;
+
+size_t bsplat_densify_workspace_bytes(int64_t N);
+/* Adds one view's statistics: for every i with max(radii[i]) > 0, grad2d[i] += |(v.x W / 2, v.y H / 2)| of
+ * v = v_means2d[i] (pixels), count[i] += 1, max_radius[i] = max(max_radius[i], max(radii[i])).  Other rows untouched.
+ * v_means2d [N, 2] and radii [N, 2] are read as 8-byte vectors (8-byte aligned). */
+int bsplat_densify_stats(int64_t N, const float* v_means2d, const int32_t* radii, int32_t width, int32_t height,
+                         float* grad2d, int32_t* count, int32_t* max_radius, void* stream);
+/* Decides every Gaussian (keep / clone / split, then prune) into the workspace (16-byte aligned, at least
+ * bsplat_densify_workspace_bytes(N), else BSPLAT_E_WORKSPACE with *needed_bytes set) and stores the totals into
+ * counts_host, a host-visible block the device writes directly: valid once the stream has reached this point. */
+int bsplat_densify_plan(int64_t N, const float* grad2d, const int32_t* count, const int32_t* max_radius,
+                        const float* log_scales, const float* opacities, const bsplat_densify_params* params,
+                        void* workspace, size_t workspace_bytes, size_t* needed_bytes,
+                        bsplat_densify_counts* counts_host, void* stream);
+/* Writes the n_out rows of every tensor from the plan in the same workspace, in one launch.  Each parent is replaced
+ * in place, in index order, by its surviving rows: kept (itself), clone (itself, then a copy), split (two children);
+ * child c of the k-th split parent in index order uses noise[k, c, 0..2] ([n_split, 2, 3]; NULL when n_split = 0).  1 to 32
+ * tensors, exactly one MEANS (src == means3d) and one LOG_SCALES (src == log_scales) among them; quats [N, 4]. */
+int bsplat_densify_apply(int64_t N, const void* workspace, const float* means3d, const float* log_scales,
+                         const float* quats, const float* noise, int32_t n_tensors,
+                         const bsplat_densify_tensor* tensors, void* stream);
 
 /* ---- stage 3, training side (SURVEY.md 8f rank 1; the reference is forward-only, render.py:11) --------- */
 /* Forward with the faithful arithmetic (kernels/rasterization.mojo:138-162) that also stores what the

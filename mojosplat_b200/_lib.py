@@ -43,6 +43,7 @@ SYMBOLS = [
     "bsplat_render_enqueue", "bsplat_rasterize_workspace_bytes", "bsplat_rasterize_fwd_train",
     "bsplat_rasterize_fwd_train_fast", "bsplat_rasterize_bwd", "bsplat_rasterize_bwd_fast", "bsplat_render_enqueue_band", "bsplat_render_enqueue_band_p2p", "bsplat_sh_eval",
     "bsplat_project_bwd", "bsplat_sh_bwd", "bsplat_ssim_workspace_bytes", "bsplat_ssim_fwd", "bsplat_ssim_bwd",
+    "bsplat_densify_workspace_bytes", "bsplat_densify_stats", "bsplat_densify_plan", "bsplat_densify_apply",
 ]
 
 
@@ -66,6 +67,22 @@ class BsplatRenderAux(Structure):
                 ("tile_ranges", c_void_p), ("sorted_ids", c_void_p), ("sorted_ids_capacity", c_int64),
                 ("n_isect", c_int64), ("timing", c_int32), ("n_launches", c_int32), ("sort_passes", c_int32),
                 ("key_bits", c_int32), ("stage_ms", c_float * 4)]
+
+
+class BsplatDensifyParams(Structure):
+    _fields_ = [("grad_threshold", c_float), ("log_clone_max_scale", c_float), ("min_opacity", c_float),
+                ("log_max_world_scale", c_float), ("max_screen_radius", c_int32), ("reserved", c_int32)]
+
+
+class BsplatDensifyTensor(Structure):
+    _fields_ = [("src", c_void_p), ("dst", c_void_p), ("width", c_int32), ("role", c_int32)]
+
+
+class BsplatDensifyCounts(Structure):
+    _fields_ = [("n_out", c_int64), ("n_clone", c_int64), ("n_split", c_int64), ("n_pruned", c_int64)]
+
+
+DENSIFY_COPY, DENSIFY_MEANS, DENSIFY_LOG_SCALES, DENSIFY_STATE = 0, 1, 2, 3
 
 
 class BsplatError(RuntimeError):
@@ -176,6 +193,18 @@ def load() -> ctypes.CDLL:
         L.bsplat_ssim_bwd.restype = ctypes.c_int
         L.bsplat_ssim_bwd.argtypes = [c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                       c_void_p]
+        L.bsplat_densify_workspace_bytes.restype = c_size_t
+        L.bsplat_densify_workspace_bytes.argtypes = [c_int64]
+        L.bsplat_densify_stats.restype = ctypes.c_int
+        L.bsplat_densify_stats.argtypes = [c_int64, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                           c_void_p]
+        L.bsplat_densify_plan.restype = ctypes.c_int
+        L.bsplat_densify_plan.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                          POINTER(BsplatDensifyParams), c_void_p, c_size_t, POINTER(c_size_t),
+                                          c_void_p, c_void_p]
+        L.bsplat_densify_apply.restype = ctypes.c_int
+        L.bsplat_densify_apply.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                           POINTER(BsplatDensifyTensor), c_void_p]
         L.bsplat_rasterize_stats.argtypes = [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                              c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
                                              c_int32, c_void_p, c_void_p, c_void_p]
