@@ -562,6 +562,198 @@ void oracle_rasterize_f64(
 }
 
 /* ------------------------------------------------------------------------------------
+ * Compositing backward in double precision, fp32 inputs: the derivative of oracle_rasterize_f64's algorithm
+ * (the decisions -- sigma >= 0, alpha >= 1/255, the 0.999 clamp, the T (1 - alpha) <= 1e-4 stop -- held fixed).
+ * Every pixel walks its tile's list front to back, stores what it composited (alpha_k, exp(-sigma_k), T_k, d_k),
+ * then walks that back to front with the upstream gradient g = grad_image[pixel]:
+ *   d out / d alpha_k = T_k (c_k . g) - (behind_k . g + T_end bg . g) / (1 - alpha_k),
+ *     behind_k = sum_{m > k} c_m alpha_m T_m;
+ *   v_sigma = -alpha_k d out / d alpha_k (zero where o exp(-sigma) > 0.999, the clamp);
+ *   colour: alpha_k T_k g;  conic: v_sigma (dx^2 / 2, dx dy, dy^2 / 2);  mean: v_sigma (a dx + b dy, b dx + c dy);
+ *   opacity: exp(-sigma_k) d out / d alpha_k (zero through the clamp);  background: T_end g.
+ * Besides the gradient, per value:
+ *   mag   the same sum with every sum and product replaced by sums and products of absolute values: the scale of
+ *         the rounding error of any evaluation order, immune to cancellation;
+ *   wmag  the same sum with each pixel's term weighted by w_pk (below), in units of 2^-22: a fp32 kernel's error
+ *         on the entry is at most rho * wmag + (fp32 additions) 2^-24 mag, rho a small multiple of 2^-22.
+ *   count the number of pixels that composited the entry (bounds the fp32 additions, atomics included).
+ * Per pixel: T_end, the last composited list index, kappa = sum alpha_k / (1 - alpha_k) (the condition number of
+ * T recovered by dividing by (1 - alpha), as both CUDA backwards do), the weight W_p and the borderline flag.
+ *
+ * Error model (the fast kernel, raster_bwd_pair_kernel, is the coarser of the two CUDA backwards; units of u = 2^-22):
+ *   alpha = 2^(L - q) with L = lg2.approx(o) (absolute error <= u), q from the log2-folded record by a chain of three
+ *   fp32 FMAs (absolute error <= 4 2^-24 (A dx^2 + |B dx dy| + C dy^2 + |L|) = u log2e (s + |ln o|),
+ *   s = a dx^2 / 2 + |b dx dy| + c dy^2 / 2), ex2.approx relative error <= u: the relative error of alpha is
+ *     e_k u,  e_k = 2 + s_k + |ln o_k|   (ln2 (1 + s + |ln o|) + 1 <= e).
+ *   The generic kernel (expf <= 2 ulp, separately rounded products) errs by <= 2^-24 (4 s + 5) <= e_k u as well.
+ *   A relative error eps of alpha_j moves T past it by eps alpha_j / (1 - alpha_j); every step of the forward product
+ *   and of the backward recovery (1 - alpha, rcp.approx or IEEE division, the product) adds <= u.  The forward and the
+ *   backward each do that once, so the relative error of any recovered T_k, and of T_end, is at most
+ *     W_p u,  W_p = sum_j (2 e_j alpha_j / (1 - alpha_j) + 2) + max_j e_j
+ *   (the max covers the alphas inside behind_k), and a term of entry k carries at most w_pk = 2 e_k + W_p units:
+ *   its own alpha enters at most twice (alpha and the factor 1 / (1 - alpha) of d out / d alpha, whose amplification
+ *   alpha / (1 - alpha) is already in W_p), and each of the ~10 fp32 products of a term adds < 1/4 u.
+ * Borderline flag: set when a decision lies within twice that error of its threshold, compared in log space (the
+ *   error is an absolute error of the exponent: for far-away Gaussians e_k u can exceed 1 while alpha is 0 on both
+ *   sides) --
+ *   |ln(255 alpha)| <= 2 e_k u;  |ln(o exp(-sigma) / 0.999)| <= 2 e_k u;  |sigma| <= 2 u s_k (s_k > 0);
+ *   |ln(T (1 - alpha) / 1e-4)| <= 2 W u, W the weight of the entries up to and including this one.
+ * With mask_borderline set, flagged pixels get g = 0 (the backward is linear in g: their terms vanish exactly).
+ * Outputs (zeroed here): grad / mag / wmag [N, 6 + C] columns (mean x, y, conic a, b, c, colour 0..C-1, opacity);
+ * count [N]; bg [3, C] (grad, mag, wmag); final_T, kappa, weight [H, W]; last_idx [H, W]; border [H, W].
+ * Accumulation: per tile into per-list-entry partials, then one omp atomic per entry and value.
+ * ---------------------------------------------------------------------------------- */
+typedef struct {
+    int32_t k;
+    int clamped;
+    double alpha, vis, T, dx, dy, e;
+} bwd_entry_t;
+
+#define BWD_U (1.0 / 4194304.0) /* 2^-22 */
+
+void oracle_raster_bwd_f64(
+    int64_t N, int CDIM, const float* means2d, const float* conics, const float* colors,
+    const float* opacities, const float* background, const int32_t* tile_ranges,
+    const int32_t* sorted_ids, int W, int H, int tile_size, const float* grad_image, int mask_borderline,
+    double* grad, double* mag, double* wmag, int64_t* count, double* bg,
+    double* final_T, int32_t* last_idx, double* kappa, double* weight, uint8_t* border)
+{
+    const int tiles_w = (W + tile_size - 1) / tile_size, tiles_h = (H + tile_size - 1) / tile_size;
+    const int V = 6 + CDIM;
+    const int S = 3 * V + 1; /* per list entry: grad[V], mag[V], wmag[V], count */
+    if (CDIM < 1 || CDIM > 16) return;
+    memset(grad, 0, sizeof(double) * (size_t)N * V);
+    memset(mag, 0, sizeof(double) * (size_t)N * V);
+    memset(wmag, 0, sizeof(double) * (size_t)N * V);
+    memset(count, 0, sizeof(int64_t) * (size_t)N);
+    memset(bg, 0, sizeof(double) * 3 * (size_t)CDIM);
+#pragma omp parallel for schedule(dynamic, 1)
+    for (int t = 0; t < tiles_w * tiles_h; ++t) {
+        const int tr = t / tiles_w, tc = t % tiles_w;
+        const int32_t r0 = tile_ranges[2 * t], r1 = tile_ranges[2 * t + 1];
+        const int64_t len = r1 > r0 ? (int64_t)(r1 - r0) : 0;
+        double* loc = (double*)calloc((size_t)(len > 0 ? len : 1) * S, sizeof(double));
+        bwd_entry_t* ent = (bwd_entry_t*)malloc(sizeof(bwd_entry_t) * (size_t)(len > 0 ? len : 1));
+        double bg_loc[3 * 16];
+        double gp[16], gabs[16];
+        for (int q = 0; q < 3 * CDIM; ++q) bg_loc[q] = 0.0;
+        for (int ii = 0; ii < tile_size; ++ii) {
+            const int i = tr * tile_size + ii;
+            if (i >= H) break;
+            for (int jj = 0; jj < tile_size; ++jj) {
+                const int j = tc * tile_size + jj;
+                if (j >= W) break;
+                const int64_t pix = (int64_t)i * W + j;
+                const double px = (double)j + 0.5, py = (double)i + 0.5;
+                /* forward walk: what the pixel composites, and how close each decision is to its threshold */
+                double T = 1.0, kap = 0.0, Wrun = 0.0, emax = 0.0;
+                int nent = 0, flag = 0;
+                int32_t last = -1;
+                for (int32_t k = r0; k < r1; ++k) {
+                    const int32_t g = sorted_ids[k];
+                    if (g < 0 || g >= N) continue;
+                    const double dx = (double)means2d[2 * g] - px, dy = (double)means2d[2 * g + 1] - py;
+                    const double a = conics[3 * g], b = conics[3 * g + 1], cc = conics[3 * g + 2];
+                    const double sigma = 0.5 * (a * dx * dx + cc * dy * dy) + b * dx * dy;
+                    const double s = 0.5 * fabs(a) * dx * dx + fabs(b * dx * dy) + 0.5 * fabs(cc) * dy * dy;
+                    const double o = opacities[g];
+                    const double vis = exp(-sigma);
+                    const double araw = o * vis;
+                    const double alpha = araw > 0.999 ? 0.999 : araw;
+                    const double e = 2.0 + s + (o > 0.0 ? fabs(log(o)) : 0.0);
+                    if (s > 0.0 && fabs(sigma) <= 2.0 * BWD_U * s) flag = 1;
+                    if (fabs(log(alpha * 255.0)) <= 2.0 * e * BWD_U) flag = 1;
+                    if (sigma < 0.0 || alpha < (1.0 / 255.0)) continue;
+                    if (fabs(log(araw / 0.999)) <= 2.0 * e * BWD_U) flag = 1;
+                    const double next_T = T * (1.0 - alpha);
+                    const double Wnext = Wrun + 2.0 * e * alpha / (1.0 - alpha) + 2.0;
+                    if (fabs(log(next_T / 1e-4)) <= 2.0 * Wnext * BWD_U) flag = 1;
+                    if (next_T <= 1e-4) break;
+                    bwd_entry_t* en = &ent[nent++];
+                    en->k = k; en->clamped = araw > 0.999; en->alpha = alpha; en->vis = vis; en->T = T;
+                    en->dx = dx; en->dy = dy; en->e = e;
+                    kap += alpha / (1.0 - alpha);
+                    Wrun = Wnext;
+                    if (e > emax) emax = e;
+                    T = next_T;
+                    last = k;
+                }
+                const double Wp = Wrun + emax;
+                final_T[pix] = T; last_idx[pix] = last; kappa[pix] = kap; weight[pix] = Wp;
+                border[pix] = (uint8_t)flag;
+                const int zero = mask_borderline && flag;
+                double bg_dot = 0.0, bg_abs = 0.0;
+                for (int c = 0; c < CDIM; ++c) {
+                    gp[c] = zero ? 0.0 : (double)grad_image[pix * CDIM + c];
+                    gabs[c] = fabs(gp[c]);
+                    bg_dot += (double)background[c] * gp[c];
+                    bg_abs += fabs((double)background[c] * gp[c]);
+                    bg_loc[c] += T * gp[c];
+                    bg_loc[CDIM + c] += T * gabs[c];
+                    bg_loc[2 * CDIM + c] += (2.0 + Wp) * T * gabs[c];
+                }
+                /* backward walk */
+                double behind = 0.0, behind_abs = 0.0;
+                for (int n = nent - 1; n >= 0; --n) {
+                    const bwd_entry_t* en = &ent[n];
+                    const int32_t g = sorted_ids[en->k];
+                    const float* col = colors + (int64_t)g * CDIM;
+                    const double a = conics[3 * g], b = conics[3 * g + 1], cc = conics[3 * g + 2];
+                    const double Tk = en->T, al = en->alpha, ra = 1.0 / (1.0 - al), fac = al * Tk;
+                    const double dx = en->dx, dy = en->dy;
+                    double cg = 0.0, cg_abs = 0.0;
+                    for (int c = 0; c < CDIM; ++c) {
+                        cg += (double)col[c] * gp[c];
+                        cg_abs += fabs((double)col[c] * gp[c]);
+                    }
+                    const double v_alpha = Tk * cg - (behind + T * bg_dot) * ra;
+                    const double m_alpha = Tk * cg_abs + (behind_abs + T * bg_abs) * ra;
+                    double gv[6 + 16], mv[6 + 16];
+                    for (int q = 0; q < V; ++q) gv[q] = mv[q] = 0.0;
+                    for (int c = 0; c < CDIM; ++c) { gv[5 + c] = fac * gp[c]; mv[5 + c] = fac * gabs[c]; }
+                    if (!en->clamped) {
+                        const double vs = -al * v_alpha, ms = al * m_alpha;
+                        gv[0] = vs * (a * dx + b * dy);       mv[0] = ms * (fabs(a * dx) + fabs(b * dy));
+                        gv[1] = vs * (b * dx + cc * dy);      mv[1] = ms * (fabs(b * dx) + fabs(cc * dy));
+                        gv[2] = 0.5 * vs * dx * dx;           mv[2] = 0.5 * ms * dx * dx;
+                        gv[3] = vs * dx * dy;                 mv[3] = ms * fabs(dx * dy);
+                        gv[4] = 0.5 * vs * dy * dy;           mv[4] = 0.5 * ms * dy * dy;
+                        gv[5 + CDIM] = en->vis * v_alpha;     mv[5 + CDIM] = en->vis * m_alpha;
+                    }
+                    const double w = 2.0 * en->e + Wp;
+                    double* L = loc + (int64_t)(en->k - r0) * S;
+                    for (int q = 0; q < V; ++q) { L[q] += gv[q]; L[V + q] += mv[q]; L[2 * V + q] += w * mv[q]; }
+                    L[3 * V] += 1.0;
+                    behind += fac * cg;
+                    behind_abs += fac * cg_abs;
+                }
+            }
+        }
+        for (int64_t k = 0; k < len; ++k) {
+            const double* L = loc + k * S;
+            if (L[3 * V] == 0.0) continue;
+            const int64_t g = sorted_ids[r0 + k];
+            for (int q = 0; q < V; ++q) {
+#pragma omp atomic
+                grad[g * V + q] += L[q];
+#pragma omp atomic
+                mag[g * V + q] += L[V + q];
+#pragma omp atomic
+                wmag[g * V + q] += L[2 * V + q];
+            }
+#pragma omp atomic
+            count[g] += (int64_t)L[3 * V];
+        }
+        for (int q = 0; q < 3 * CDIM; ++q) {
+#pragma omp atomic
+            bg[q] += bg_loc[q];
+        }
+        free(loc);
+        free(ent);
+    }
+}
+
+/* ------------------------------------------------------------------------------------
  * Outlier audit (SURVEY H4).  The alpha >= 1/255 test and the T (1 - alpha) <= 1e-4 stop make a pixel
  * discontinuous in exp(): two correct fp32 implementations may take a different branch when a value sits
  * within rounding distance of a threshold, and the pixel then differs by up to alpha T colour.  That is the

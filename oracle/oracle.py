@@ -163,6 +163,47 @@ def rasterize_f64(means2d, conics, colors, opacities, background, tile_ranges, s
     return image
 
 
+def raster_bwd_f64(means2d, conics, colors, opacities, background, tile_ranges, sorted_ids, W, H, tile_size,
+                   grad_image, mask_borderline=False):
+    """Compositing backward in double precision on the fp32 inputs (see oracle.c: oracle_raster_bwd_f64), for the
+    upstream gradient grad_image [H, W, C].  Returns a dict of numpy arrays:
+      grad_means2d [N,2], grad_conics [N,3], grad_colors [N,C], grad_opacities [N], grad_background [C];
+      mag_* (sums of absolute values of the same terms) and wmag_* (the same, each pixel's term weighted by the
+      rounding-error weight of oracle.c, in units of 2^-22), same shapes;
+      count [N] (pixels that composited each Gaussian); final_T, kappa, weight [H,W] float64; last_idx [H,W] int32
+      (last composited list index, -1 if none); borderline [H,W] bool.
+    mask_borderline=True differentiates with grad_image zeroed on the borderline pixels."""
+    means2d, conics, colors = _f32(means2d), _f32(conics), _f32(colors)
+    opacities = _f32(opacities).reshape(-1)
+    background = _f32(background).reshape(-1)
+    N, C = colors.shape
+    assert 1 <= C <= 16
+    ranges = np.ascontiguousarray(np.asarray(tile_ranges, dtype=np.int32))
+    ids = np.ascontiguousarray(np.asarray(sorted_ids, dtype=np.int32))
+    gimg = _f32(grad_image).reshape(H, W, C)
+    V = 6 + C
+    grad, mag, wmag = (np.empty((N, V), np.float64) for _ in range(3))
+    count = np.empty((N,), np.int64)
+    bg = np.empty((3, C), np.float64)
+    final_T, kappa, weight = (np.empty((H, W), np.float64) for _ in range(3))
+    last_idx = np.empty((H, W), np.int32)
+    border = np.empty((H, W), np.uint8)
+    lib().oracle_raster_bwd_f64(ctypes.c_int64(N), ctypes.c_int(C), _ptr(means2d), _ptr(conics), _ptr(colors),
+                                _ptr(opacities), _ptr(background), _ptr(ranges), _ptr(ids), ctypes.c_int(W),
+                                ctypes.c_int(H), ctypes.c_int(tile_size), _ptr(gimg),
+                                ctypes.c_int(int(mask_borderline)), _ptr(grad), _ptr(mag), _ptr(wmag), _ptr(count), _ptr(bg), _ptr(final_T),
+                                _ptr(last_idx), _ptr(kappa), _ptr(weight), _ptr(border))
+    out = dict(count=count, final_T=final_T, last_idx=last_idx, kappa=kappa, weight=weight,
+               borderline=border.astype(bool))
+    for pre, arr, b in (("grad", grad, bg[0]), ("mag", mag, bg[1]), ("wmag", wmag, bg[2])):
+        out[f"{pre}_means2d"] = arr[:, 0:2].copy()
+        out[f"{pre}_conics"] = arr[:, 2:5].copy()
+        out[f"{pre}_colors"] = arr[:, 5:5 + C].copy()
+        out[f"{pre}_opacities"] = arr[:, 5 + C].copy()
+        out[f"{pre}_background"] = b.copy()
+    return out
+
+
 def raster_audit(means2d, conics, colors, opacities, background, tile_ranges, sorted_ids, W, H, tile_size,
                  pixels, observed, atol=1e-4, rtol=1e-4, rel_window=1e-4):
     """SURVEY H4 audit of out-of-tolerance pixels (see oracle.c: oracle_raster_audit).

@@ -73,6 +73,28 @@ def image_gate(img, ref, frac_allowed=1e-4, atol=1e-4, rtol=1e-4, max_err_allowe
     return res
 
 
+# rho of the per-entry backward bound (oracle.c: oracle_raster_bwd_f64), from the kernels' arithmetic: 2 x 2^-22 for the
+# pair kernel (ex2.approx, lg2.approx, rcp.approx), 4 x 2^-24 for the generic kernel (libdevice expf, IEEE division)
+BWD_RHO = {"fast": 2.0 * 2.0 ** -22, "faithful": 4.0 * 2.0 ** -24}
+BWD_GRADS = ["means2d", "conics", "colors", "opacities", "background"]
+
+
+def bwd_entry_ratios(got, ref, rho, n_pixels):
+    """err / bound of every gradient entry against oracle.raster_bwd_f64's result `ref`:
+    |got - ref| <= rho wmag + n_e 2^-24 mag + 1e-12, n_e the pixels that composited the Gaussian (for the background
+    gradient, a torch reduction over the image: n_pixels)."""
+    out = {}
+    for n in BWD_GRADS:
+        if n not in got:
+            continue
+        cnt = float(n_pixels) if n == "background" else ref["count"].astype(np.float64)
+        if n in ("means2d", "conics", "colors"):
+            cnt = cnt[:, None]
+        bound = rho * ref[f"wmag_{n}"] + cnt * 2.0 ** -24 * ref[f"mag_{n}"] + 1e-12
+        out[n] = np.abs(np.asarray(got[n], np.float64) - ref[f"grad_{n}"]) / bound
+    return out
+
+
 def audit_inputs(ref, sc, tile_size=16):
     """Raster inputs of an oracle.render(..., return_all=True) result, for image_gate(audit=...)."""
     return dict(means2d=ref["means2d"], conics=ref["conics"], colors=sc.colors.numpy(), opacities=sc.opacities.numpy(),

@@ -10,7 +10,7 @@ import pytest
 import torch
 
 import mojosplat_b200 as ms
-from helpers import dev, image_gate
+from helpers import BWD_RHO, bwd_entry_ratios, dev, image_gate
 from mojosplat_b200 import rasterization
 from oracle import oracle
 
@@ -106,6 +106,26 @@ def _check_backward(cuda_device, N, HW, ts, C, seed, mode):
         # fp32 compositing + atomics vs fp64 autograd: 1e-3 of the largest entry, plus 1e-3 relative
         np.testing.assert_allclose(got, want, atol=1e-3 * scale, rtol=1e-3, err_msg=name)
         assert np.abs(want).max() > 0 or N == 0, name
+    rho = BWD_RHO["fast" if (mode == "fast" and ts == 16 and C == 3) else "faithful"]
+    _assert_every_entry(cuda_device, (m2, con, c, o, bg), ranges, ids, cam, ts, mode, gimg.numpy(), rho)
+
+
+def _assert_every_entry(cuda_device, inputs, ranges, ids, cam, ts, mode, gimg, rho):
+    """Every gradient entry within the per-entry bound against the fp64 reference (oracle.raster_bwd_f64), with the
+    upstream gradient zeroed on the reference's borderline pixels (on both sides)."""
+    m2, con, c, o, bg = inputs
+    H, W = int(cam.H), int(cam.W)
+    ref = oracle.raster_bwd_f64(m2, con, c, o, bg, ranges, ids, W, H, ts, gimg, mask_borderline=True)
+    gm = np.where(ref["borderline"][..., None], np.float32(0), gimg.astype(np.float32))
+    t32 = [dev(x, cuda_device).requires_grad_(True) for x in inputs]
+    img = rasterization.rasterize_gaussians_diff(*t32, dev(ranges, cuda_device), dev(ids, cuda_device), cam, ts,
+                                                 mode=mode)
+    img.backward(dev(gm, cuda_device))
+    got = {n: x.grad.cpu().double().numpy() for n, x in zip(["means2d", "conics", "colors", "opacities",
+                                                             "background"], t32)}
+    assert float(ref["borderline"].mean()) <= 0.05
+    for n, r in bwd_entry_ratios(got, ref, rho, H * W).items():
+        assert r.max() <= 1.0, (n, float(r.max()), np.unravel_index(int(r.argmax()), r.shape))
 
 
 def test_train_forward_equals_faithful_kernel(cuda_device):
@@ -210,6 +230,10 @@ def test_backward_saturated_pixels_and_clamp(cuda_device, mode):
     for a, b in zip(t32, t64):
         want = b.grad.numpy(); scale = np.abs(want).max() + 1e-12
         np.testing.assert_allclose(a.grad.cpu().double().numpy(), want, atol=2e-3 * scale, rtol=2e-3)
+    rho = BWD_RHO[mode]
+    for gimg in (np.ones((HW, HW, 3), np.float32),
+                 torch.randn(HW, HW, 3, generator=torch.Generator().manual_seed(12)).numpy()):
+        _assert_every_entry(cuda_device, (m2, con, c, o, bg), ranges, ids, cam, 16, mode, gimg, rho)
     # Gaussians that autograd says never contributed (behind saturated pixels everywhere) get exactly zero
     never = (t64[2].grad.abs().sum(dim=1) == 0).numpy()
     assert float(t32[2].grad.cpu()[torch.from_numpy(never)].abs().sum()) == 0.0
