@@ -1,5 +1,6 @@
 """compute-sanitizer workload: every kernel of libbsplat.so on small scenes (both rule sets, packed layout, row bands,
-long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward, SSIM + L1 loss, densification).  Run as
+long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward, SSIM + L1 loss, densification, MCMC
+noise / relocation / sample-add).  Run as
 
     compute-sanitizer --tool memcheck  python benchmarks/sanitize.py
     compute-sanitizer --tool racecheck python benchmarks/sanitize.py
@@ -87,5 +88,14 @@ for cfg, N, sem in [("config1_1k_256", None, "cuda"), ("config3_1m_1080p", 8000 
     dopt.step()
     dnew, dcounts = ms.densify_and_prune(dp, st, 1.0, min_opacity=0.3, optimizer=dopt)
     assert dcounts["n_out"] == dnew["sh"].shape[0] > 0
+    # MCMC densification: noise, relocation (in place, Adam state zeroed) and sample-add (out of place)
+    mp = {k: v.detach().clone().requires_grad_(True) for k, v in dnew.items()}
+    mopt = torch.optim.Adam(list(mp.values()))
+    for v in mp.values():
+        v.grad = torch.ones_like(v)
+    mopt.step()
+    ms.mcmc_inject_noise(mp, 1e3)
+    mnew, mcounts = ms.mcmc_refine(mp, cap_max=2 * dcounts["n_out"], min_opacity=0.5, optimizer=mopt)
+    assert mcounts["n_relocated"] > 0 and mcounts["n_out"] == mnew["sh"].shape[0] > dcounts["n_out"]
     torch.cuda.synchronize()
     print(cfg, sem, "ok", float(img.mean()), flush=True)

@@ -32,6 +32,8 @@
  *                             L1 on one image pair, forward + backward), checked against torch autograd
  *   bsplat_densify_stats / _plan / _apply   no reference counterpart: adaptive density control (3DGS's gradient
  *                             statistics and densify_and_prune), checked against a torch restatement
+ *   bsplat_mcmc_noise / _relocate / _add   no reference counterpart: 3DGS-MCMC densification (position noise,
+ *                             relocation, sample-add), checked against a torch restatement
  *   bsplat_render_fwd         mojosplat/render.py:12-103 render_gaussians (the three stages chained
  *                              on one stream with a single 16-byte read-back)
  *   bsplat_render_enqueue     same without the read-back (device-side M, two-stream overlap, graph capture)
@@ -306,6 +308,49 @@ int bsplat_densify_plan(int64_t N, const float* grad2d, const int32_t* count, co
 int bsplat_densify_apply(int64_t N, const void* workspace, const float* means3d, const float* log_scales,
                          const float* quats, const float* noise, int32_t n_tensors,
                          const bsplat_densify_tensor* tensors, void* stream);
+
+/* ---- MCMC densification (no reference counterpart) ------------------------------------------- */
+/* 3DGS-MCMC (Kheradmand et al. 2024; gsplat's MCMCStrategy).  The caller draws the indices and the noise; these entry
+ * points turn them into rows.  Opacity o is the stored value, or sigmoid of it when opacity_logits is set (then writes
+ * store log(o / (1 - o))); log-scales s; quaternions (w, x, y, z), normalised as in bsplat_project_fwd. */
+typedef struct bsplat_mcmc_params {
+    float min_opacity;       /* lower clamp of a relocated opacity */
+    int32_t opacity_logits;  /* 0: opacities as the renderer sees them, 1: logits */
+} bsplat_mcmc_params;
+/* roles of a bsplat_mcmc_tensor */
+#define BSPLAT_MCMC_COPY 0        /* copied row-wise */
+#define BSPLAT_MCMC_OPACITY 1     /* [N, 1]: relocated rows get o' = clamp(1 - (1 - o)^(1/n), min_opacity, 1 - 2^-23) */
+#define BSPLAT_MCMC_LOG_SCALES 2  /* [N, 3]: relocated rows get s + log(o / D(n, o')) */
+#define BSPLAT_MCMC_STATE 3       /* optimizer state: zeroed for relocated and new rows (see each entry point) */
+typedef struct bsplat_mcmc_tensor {
+    const float* src;  /* [N, width] */
+    float* dst;        /* bsplat_mcmc_relocate: == src (in place); bsplat_mcmc_add: [N + n_add, width], != src */
+    int32_t width;     /* 1..256 floats per row */
+    int32_t role;
+} bsplat_mcmc_tensor;
+
+/* Bytes of the workspace bsplat_mcmc_relocate / _add need for N rows (20 per row, 16-byte aligned). */
+size_t bsplat_mcmc_workspace_bytes(int64_t N);
+/* In place: means3d[i] += scale * sigmoid(100 ((1 - o_i) - 0.995)) * R_i S_i^2 R_i^T noise[i], S_i = diag(exp(s_i)),
+ * noise [N, 3] (any distribution; the strategy draws standard normals).  The gate is evaluated in double and rounded
+ * once with scale; a row whose gate times scale rounds to 0 is left untouched.  quats 16-byte aligned. */
+int bsplat_mcmc_noise(int64_t N, float* means3d, const float* log_scales, const float* quats, const float* opacities,
+                      const float* noise, float scale, const bsplat_mcmc_params* params, void* stream);
+/* Relocation, in place.  A row sampled c > 0 times in sampled[0, n_dead) (int64, in [0, N)) gets, with
+ * n = min(c + 1, 51), its opacity o' and log-scales s + log(o / D), D = sum_{k<n} C(n, k+1) (-1)^k o'^(k+1) / sqrt(k+1)
+ * (evaluated in double, rounded once); then dead row dead[k] becomes a copy of updated row sampled[k].  No dead row may
+ * be sampled.  STATE rows of sampled and dead rows are zeroed.  1 to 32 tensors, exactly one OPACITY (width 1) and one
+ * LOG_SCALES (width 3); workspace 16-byte aligned, at least bsplat_mcmc_workspace_bytes(N), else BSPLAT_E_WORKSPACE
+ * with *needed_bytes (nullable) set. */
+int bsplat_mcmc_relocate(int64_t N, int64_t n_dead, const int64_t* dead, const int64_t* sampled,
+                         const bsplat_mcmc_params* params, int32_t n_tensors, const bsplat_mcmc_tensor* tensors,
+                         void* workspace, size_t workspace_bytes, size_t* needed_bytes, void* stream);
+/* Sample-add, out of place.  The rows sampled in sampled[0, n_add) get the relocated values as above; dst row r < N is
+ * the updated source row r, dst row N + k the updated row sampled[k].  STATE rows r < N are copied, STATE rows N + k
+ * are zero.  Same descriptor and workspace rules. */
+int bsplat_mcmc_add(int64_t N, int64_t n_add, const int64_t* sampled, const bsplat_mcmc_params* params,
+                    int32_t n_tensors, const bsplat_mcmc_tensor* tensors, void* workspace, size_t workspace_bytes,
+                    size_t* needed_bytes, void* stream);
 
 /* ---- stage 3, training side (SURVEY.md 8f rank 1; the reference is forward-only, render.py:11) --------- */
 /* Forward with the faithful arithmetic (kernels/rasterization.mojo:138-162) that also stores what the

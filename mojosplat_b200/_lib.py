@@ -44,6 +44,7 @@ SYMBOLS = [
     "bsplat_rasterize_fwd_train_fast", "bsplat_rasterize_bwd", "bsplat_rasterize_bwd_fast", "bsplat_render_enqueue_band", "bsplat_render_enqueue_band_p2p", "bsplat_sh_eval",
     "bsplat_project_bwd", "bsplat_sh_bwd", "bsplat_ssim_workspace_bytes", "bsplat_ssim_fwd", "bsplat_ssim_bwd",
     "bsplat_densify_workspace_bytes", "bsplat_densify_stats", "bsplat_densify_plan", "bsplat_densify_apply",
+    "bsplat_mcmc_workspace_bytes", "bsplat_mcmc_noise", "bsplat_mcmc_relocate", "bsplat_mcmc_add",
 ]
 
 
@@ -83,6 +84,17 @@ class BsplatDensifyCounts(Structure):
 
 
 DENSIFY_COPY, DENSIFY_MEANS, DENSIFY_LOG_SCALES, DENSIFY_STATE = 0, 1, 2, 3
+
+
+class BsplatMcmcParams(Structure):
+    _fields_ = [("min_opacity", c_float), ("opacity_logits", c_int32)]
+
+
+class BsplatMcmcTensor(Structure):
+    _fields_ = [("src", c_void_p), ("dst", c_void_p), ("width", c_int32), ("role", c_int32)]
+
+
+MCMC_COPY, MCMC_OPACITY, MCMC_LOG_SCALES, MCMC_STATE = 0, 1, 2, 3
 
 
 class BsplatError(RuntimeError):
@@ -205,6 +217,17 @@ def load() -> ctypes.CDLL:
         L.bsplat_densify_apply.restype = ctypes.c_int
         L.bsplat_densify_apply.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
                                            POINTER(BsplatDensifyTensor), c_void_p]
+        L.bsplat_mcmc_workspace_bytes.restype = c_size_t
+        L.bsplat_mcmc_workspace_bytes.argtypes = [c_int64]
+        L.bsplat_mcmc_noise.restype = ctypes.c_int
+        L.bsplat_mcmc_noise.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
+                                        POINTER(BsplatMcmcParams), c_void_p]
+        L.bsplat_mcmc_relocate.restype = ctypes.c_int
+        L.bsplat_mcmc_relocate.argtypes = [c_int64, c_int64, c_void_p, c_void_p, POINTER(BsplatMcmcParams), c_int32,
+                                           POINTER(BsplatMcmcTensor), c_void_p, c_size_t, POINTER(c_size_t), c_void_p]
+        L.bsplat_mcmc_add.restype = ctypes.c_int
+        L.bsplat_mcmc_add.argtypes = [c_int64, c_int64, c_void_p, POINTER(BsplatMcmcParams), c_int32,
+                                      POINTER(BsplatMcmcTensor), c_void_p, c_size_t, POINTER(c_size_t), c_void_p]
         L.bsplat_rasterize_stats.argtypes = [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                              c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
                                              c_int32, c_void_p, c_void_p, c_void_p]

@@ -5,8 +5,9 @@ synchronisation); ``densify_and_prune`` then clones, splits and prunes the Gauss
 read-back of four counts and one gather kernel that writes every parameter and, with ``optimizer``, every Adam moment
 of the new set.  ``scene_extent`` is 3DGS's camera-extent helper.
 
-Out of scope: the opacity reset (two torch lines, see ``densify_and_prune``), AbsGS gradients, MCMC relocation, fused
-optimizers and multi-GPU densification.
+The other standard recipe, 3DGS-MCMC's relocation and sample-add under a fixed budget, is ``mcmc.py``.  Out of scope
+here: the opacity reset (two torch lines, see ``densify_and_prune``), AbsGS gradients, fused optimizers and multi-GPU
+densification.
 """
 from __future__ import annotations
 
@@ -85,6 +86,56 @@ def _log_f32(x: float) -> float:
     return float(torch.tensor(math.log(x) if x > 0 else -math.inf, dtype=torch.float64).float())
 
 
+def _row_jobs(params: dict, optimizer, N: int):
+    """Every tensor a row-wise rewrite of ``params`` touches: ``(key, None, tensor)`` for each param, then
+    ``(key, state name, tensor)`` for each optimizer state tensor with N leading rows; ``owner`` maps a param's id to its
+    key.  Raises when the optimizer holds a tensor that is not in ``params`` or the tensors do not fit the kernels'
+    descriptors (at most 32, 1..256 floats per row)."""
+    jobs = [(k, None, t) for k, t in params.items()]
+    owner = {id(t): k for k, t in params.items()}
+    if optimizer is not None:
+        for group in optimizer.param_groups:
+            for p in group["params"]:
+                if id(p) not in owner:
+                    raise ValueError("the optimizer holds a parameter that is not in params")
+                for sk, sv in optimizer.state.get(p, {}).items():
+                    if isinstance(sv, torch.Tensor) and sv.dim() >= 1 and sv.shape[0] == N:
+                        _check_cuda_f32(f"optimizer state '{sk}' of params['{owner[id(p)]}']", sv)
+                        jobs.append((owner[id(p)], sk, sv))
+    if len(jobs) > MAX_TENSORS:
+        raise ValueError(f"{len(jobs)} tensors to remap (params + optimizer state); at most {MAX_TENSORS}")
+    for k, sk, t in jobs:
+        w = math.prod(t.shape[1:])
+        if not 1 <= w <= MAX_WIDTH:
+            raise ValueError(f"params['{k}']{'' if sk is None else ' state ' + sk}: {w} values per row; "
+                             f"the gather takes 1..{MAX_WIDTH}")
+    return jobs, owner
+
+
+def _rebind(jobs, outs, owner, optimizer) -> dict:
+    """The new params (fresh leaves with ``requires_grad=True``) from the outputs of ``jobs``; with ``optimizer``, its
+    groups and state are rebound to them in place (scalar state such as ``step`` is kept)."""
+    new_params = {}
+    new_state = {}
+    for (k, sk, t), o in zip(jobs, outs):
+        if sk is None:
+            new_params[k] = o.requires_grad_(True)
+        else:
+            new_state.setdefault(k, {})[sk] = o
+    if optimizer is not None:
+        for group in optimizer.param_groups:
+            for i, old in enumerate(group["params"]):
+                k = owner[id(old)]
+                new = new_params[k]
+                group["params"][i] = new
+                st = optimizer.state.pop(old, None)
+                if st is not None:
+                    st = dict(st)
+                    st.update(new_state.get(k, {}))
+                    optimizer.state[new] = st
+    return new_params
+
+
 def densify_and_prune(params: dict, stats: DensifyStats, scene_extent: float, *, opacities=None,
                       grad_threshold: float = 2e-4, percent_dense: float = 0.01, min_opacity: float = 0.005,
                       max_screen_radius=None, max_world_scale=None, optimizer=None, generator=None):
@@ -148,25 +199,7 @@ def densify_and_prune(params: dict, stats: DensifyStats, scene_extent: float, *,
     if opacities.numel() != N or opacities.device != dev:
         raise ValueError(f"opacities must hold N = {N} values on the params' device")
 
-    # every tensor the gather writes: the params, then the optimizer state with N leading rows
-    jobs = [(k, None, t) for k, t in params.items()]
-    owner = {id(t): k for k, t in params.items()}
-    if optimizer is not None:
-        for group in optimizer.param_groups:
-            for p in group["params"]:
-                if id(p) not in owner:
-                    raise ValueError("the optimizer holds a parameter that is not in params")
-                for sk, sv in optimizer.state.get(p, {}).items():
-                    if isinstance(sv, torch.Tensor) and sv.dim() >= 1 and sv.shape[0] == N:
-                        _check_cuda_f32(f"optimizer state '{sk}' of params['{owner[id(p)]}']", sv)
-                        jobs.append((owner[id(p)], sk, sv))
-    if len(jobs) > MAX_TENSORS:
-        raise ValueError(f"{len(jobs)} tensors to remap (params + optimizer state); at most {MAX_TENSORS}")
-    for k, sk, t in jobs:
-        w = math.prod(t.shape[1:])
-        if not 1 <= w <= MAX_WIDTH:
-            raise ValueError(f"params['{k}']{'' if sk is None else ' state ' + sk}: {w} values per row; "
-                             f"the gather takes 1..{MAX_WIDTH}")
+    jobs, owner = _row_jobs(params, optimizer, N)
 
     L = _lib.require_device(dev)
     p = _lib.BsplatDensifyParams()
@@ -199,23 +232,6 @@ def densify_and_prune(params: dict, stats: DensifyStats, scene_extent: float, *,
             rc = L.bsplat_densify_apply(N, _lib.ptr(ws), _lib.ptr(means), _lib.ptr(scales), _lib.ptr(quats),
                                         _lib.ptr(noise), len(jobs), desc, stream)
             _lib.check(rc, "bsplat_densify_apply")
-    new_params = {}
-    new_state = {}
-    for (k, sk, t), o in zip(jobs, outs):
-        if sk is None:
-            new_params[k] = o.requires_grad_(True)
-        else:
-            new_state.setdefault(k, {})[sk] = o
-    if optimizer is not None:
-        for group in optimizer.param_groups:
-            for i, old in enumerate(group["params"]):
-                k = owner[id(old)]
-                new = new_params[k]
-                group["params"][i] = new
-                st = optimizer.state.pop(old, None)
-                if st is not None:
-                    st = dict(st)
-                    st.update(new_state.get(k, {}))
-                    optimizer.state[new] = st
+    new_params = _rebind(jobs, outs, owner, optimizer)
     stats.reset(n_out)
     return new_params, dict(n_out=n_out, n_clone=n_clone, n_split=n_split, n_pruned=n_pruned)
