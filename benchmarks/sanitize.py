@@ -1,6 +1,6 @@
 """compute-sanitizer workload: every kernel of libbsplat.so on small scenes (both rule sets, packed layout, row bands,
-long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward, SSIM + L1 loss, densification, MCMC
-noise / relocation / sample-add).  Run as
+long-list pre-pass, sync-free / captured frames, backward with and without the absolute mean gradient, SH, projection /
+SH backward, SSIM + L1 loss, densification, MCMC noise / relocation / sample-add).  Run as
 
     compute-sanitizer --tool memcheck  python benchmarks/sanitize.py
     compute-sanitizer --tool racecheck python benchmarks/sanitize.py
@@ -49,6 +49,12 @@ for cfg, N, sem in [("config1_1k_256", None, "cuda"), ("config3_1m_1080p", 8000 
         out = rasterization.rasterize_gaussians_diff(*t, bg, aux["tile_ranges"], aux["sorted_ids"], sc.camera, 16,
                                                      mode=mode)
         out.sum().backward()
+        # ... and their AbsGS instantiations (bsplat_rasterize_bwd[_fast]_abs)
+        absgrad = torch.zeros_like(aux["means2d"])
+        out = rasterization.rasterize_gaussians_diff(*t, bg, aux["tile_ranges"], aux["sorted_ids"], sc.camera, 16,
+                                                     mode=mode, means2d_absgrad=absgrad)
+        out.sum().backward()
+        assert bool(torch.isfinite(absgrad).all()) and bool((absgrad >= 0).all())
     pipe = OverlappedPipeline(dev, sc.N, sc.camera.W, sc.camera.H, semantics=semv, m_capacity=200 * sc.N + 4096)
     cams = synthetic.orbit_cameras(4, sc.camera.W, sc.camera.H, sc.camera.fx)
     pipe.render(*g, cams, bg); pipe.check()

@@ -1,7 +1,8 @@
 """Memory-safety and race evidence without compute-sanitizer (closed on some pools; see profiles/*sanitize*):
 
   1. the whole kernel inventory (benchmarks/sanitize.py: both rule sets, packed layout, row bands with and without the
-     band pre-test, long-list pre-pass, sync-free / captured frames, backward, SH, projection / SH backward) runs under
+     band pre-test, long-list pre-pass, sync-free / captured frames, backward with and without the absolute mean
+     gradient, SH, projection / SH backward) runs under
      the CHECKED build
      (`make -C mojosplat_b200/csrc checked`: device-side bounds / invariant checks, BSPLAT_DASSERT) -- a failed check
      traps and the CUDA error surfaces here;

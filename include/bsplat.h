@@ -383,6 +383,17 @@ int bsplat_rasterize_bwd(int64_t N, int32_t channels, const float* means2d, cons
                          int32_t width, int32_t height, int32_t tile_size, const float* final_T,
                          const int32_t* last_idx, const float* grad_image, float* grad_means2d,
                          float* grad_conics, float* grad_colors, float* grad_opacities, void* stream);
+/* The same, and ACCUMULATES AbsGS's absolute screen-space gradient into the caller-zeroed grad_means2d_abs[N,2]:
+ * per Gaussian, the sum over the pixels it was composited at of |d loss_p / d means2d| (x and y separately, the
+ * absolute value taken per pixel; gsplat's `absgrad`). grad_means2d_abs must not be NULL when N > 0; every other
+ * rule is bsplat_rasterize_bwd's. */
+int bsplat_rasterize_bwd_abs(int64_t N, int32_t channels, const float* means2d, const float* conics,
+                             const float* colors, const float* opacities, const float* background,
+                             const int32_t* tile_ranges, const int32_t* sorted_ids, int64_t M,
+                             int32_t width, int32_t height, int32_t tile_size, const float* final_T,
+                             const int32_t* last_idx, const float* grad_image, float* grad_means2d,
+                             float* grad_means2d_abs, float* grad_conics, float* grad_colors,
+                             float* grad_opacities, void* stream);
 
 /* ---- fused forward ------------------------------------------------------------------------- */
 /* Optional outputs of the fused path (any pointer may be NULL). */
@@ -490,6 +501,14 @@ int bsplat_rasterize_bwd_fast(int64_t N, const float* means2d, const float* coni
                               int32_t height, const float* final_T, const int32_t* last_idx,
                               const float* grad_image, float* grad_means2d, float* grad_conics, float* grad_colors,
                               float* grad_opacities, void* workspace, size_t workspace_bytes, void* stream);
+/* bsplat_rasterize_bwd_fast plus the absolute screen-space gradient, as bsplat_rasterize_bwd_abs. */
+int bsplat_rasterize_bwd_fast_abs(int64_t N, const float* means2d, const float* conics, const float* colors,
+                                  const float* opacities, const float* background, const int32_t* tile_ranges,
+                                  const int32_t* tile_order, const int32_t* sorted_ids, int64_t M, int32_t width,
+                                  int32_t height, const float* final_T, const int32_t* last_idx,
+                                  const float* grad_image, float* grad_means2d, float* grad_means2d_abs,
+                                  float* grad_conics, float* grad_colors, float* grad_opacities, void* workspace,
+                                  size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

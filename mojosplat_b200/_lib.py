@@ -41,7 +41,8 @@ SYMBOLS = [
     "bsplat_render_fwd_host", "bsplat_microbench", "bsplat_bin2_workspace_bytes", "bsplat_bin2_prepare",
     "bsplat_bin2_finish", "bsplat_tile_order", "bsplat_render_begin", "bsplat_render_end",
     "bsplat_render_enqueue", "bsplat_rasterize_workspace_bytes", "bsplat_rasterize_fwd_train",
-    "bsplat_rasterize_fwd_train_fast", "bsplat_rasterize_bwd", "bsplat_rasterize_bwd_fast", "bsplat_render_enqueue_band", "bsplat_render_enqueue_band_p2p", "bsplat_sh_eval",
+    "bsplat_rasterize_fwd_train_fast", "bsplat_rasterize_bwd", "bsplat_rasterize_bwd_fast", "bsplat_rasterize_bwd_abs",
+    "bsplat_rasterize_bwd_fast_abs", "bsplat_render_enqueue_band", "bsplat_render_enqueue_band_p2p", "bsplat_sh_eval",
     "bsplat_project_bwd", "bsplat_sh_bwd", "bsplat_ssim_workspace_bytes", "bsplat_ssim_fwd", "bsplat_ssim_bwd",
     "bsplat_densify_workspace_bytes", "bsplat_densify_stats", "bsplat_densify_plan", "bsplat_densify_apply",
     "bsplat_mcmc_workspace_bytes", "bsplat_mcmc_noise", "bsplat_mcmc_relocate", "bsplat_mcmc_add",
@@ -171,6 +172,14 @@ def load() -> ctypes.CDLL:
                                                 c_void_p, c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p,
                                                 c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                                 c_void_p]
+        L.bsplat_rasterize_bwd_abs.argtypes = [c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                               c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_void_p,
+                                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                               c_void_p]
+        L.bsplat_rasterize_bwd_fast_abs.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                    c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32,
+                                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                    c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
         L.bsplat_rasterize_workspace_bytes.restype = c_size_t
         L.bsplat_rasterize_workspace_bytes.argtypes = [c_int64]
         L.bsplat_tile_order.argtypes = [c_int32, c_int32, c_void_p, c_void_p, c_void_p]

@@ -21,6 +21,9 @@
 //                            batch; per Gaussian the 6 + C partial gradients are reduced over the warp
 //                            (butterfly shuffles, skipped when no lane of the warp contributes) and added
 //                            to the per-Gaussian gradient arrays with one atomic per value and warp.
+//   Both backward kernels also come with kAbs = true (bsplat_rasterize_bwd[_fast]_abs): per Gaussian they then add the
+//   sum over pixels of |d loss_p / d mean| (AbsGS's densification statistic, gsplat's absgrad; the absolute value taken
+//   per pixel) into a second [N, 2] array.  kAbs = false is the plain kernel, instruction for instruction.
 //   d out / d alpha_k = c_k T_k - (sum_{m>k} c_m alpha_m T_m + T_end bg) / (1 - alpha_k)
 //   d alpha / d sigma = -alpha, d alpha / d o = exp(-sigma)        (zero through the 0.999 clamp)
 //   d sigma / d(a, b, c) = (0.5 dx^2, dx dy, 0.5 dy^2),  d sigma / d mean = (a dx + b dy, b dx + c dy)
@@ -44,13 +47,13 @@ __device__ __forceinline__ void tile_pixel_of(const int tid, const int ts, int& 
     }
 }
 
-// Warp reduction of P (8 or 16) values per lane in P + log2(32 / P) shuffles instead of 5 P: at every step a lane keeps
-// one half of its values and sends the other half to its partner, so the sums end up SPREAD over the lanes --
-// lane L holds the total of value (L >> (P == 16 ? 1 : 2)) in v[0] -- and P lanes can issue their atomics in one
-// instruction instead of one lane issuing P.
+// Warp reduction of P (4, 8 or 16) values per lane in P + log2(32 / P) shuffles instead of 5 P: at every step a lane
+// keeps one half of its values and sends the other half to its partner, so the sums end up SPREAD over the lanes --
+// lane L holds the total of value L / (32 / P) in v[0] -- and P lanes can issue their atomics in one instruction
+// instead of one lane issuing P.
 template <int P>
 __device__ __forceinline__ void warp_reduce_spread(float (&v)[P], const unsigned lane) {
-    static_assert(P == 8 || P == 16, "8 or 16 values");
+    static_assert(P == 4 || P == 8 || P == 16, "4, 8 or 16 values");
     int d = 16;
 #pragma unroll
     for (int half = P / 2; half >= 1; half >>= 1, d >>= 1) {
@@ -175,7 +178,7 @@ raster_train_fwd_kernel(const int64_t N, const float* __restrict__ means2d, cons
     }
 }
 
-template <int CH>
+template <int CH, bool kAbs>
 __global__ void __launch_bounds__(1024)
 raster_bwd_kernel(const int64_t N, const float* __restrict__ means2d, const float* __restrict__ conics,
                   const float* __restrict__ colors, const float* __restrict__ opacities,
@@ -183,7 +186,8 @@ raster_bwd_kernel(const int64_t N, const float* __restrict__ means2d, const floa
                   const int32_t* __restrict__ sorted_ids, const int W, const int H, const int ts,
                   const int tiles_w, const float* __restrict__ final_T, const int32_t* __restrict__ last_idx,
                   const float* __restrict__ grad_image, float* __restrict__ g_means2d,
-                  float* __restrict__ g_conics, float* __restrict__ g_colors, float* __restrict__ g_opac) {
+                  float* __restrict__ g_conics, float* __restrict__ g_colors, float* __restrict__ g_opac,
+                  float* __restrict__ g_means2d_abs) {
     extern __shared__ float s_buf[];
     const int nthreads = blockDim.x;
     float* s_mx = s_buf;
@@ -291,7 +295,7 @@ raster_bwd_kernel(const int64_t N, const float* __restrict__ means2d, const floa
             }
             if (!__any_sync(0xffffffffu, valid)) continue;  // nothing to reduce for this warp
             float v_rgb[CH];
-            float v_ca = 0.f, v_cb = 0.f, v_cc = 0.f, v_mx = 0.f, v_my = 0.f, v_op = 0.f;
+            float v_ca = 0.f, v_cb = 0.f, v_cc = 0.f, v_mx = 0.f, v_my = 0.f, v_op = 0.f, v_ax = 0.f, v_ay = 0.f;
 #pragma unroll
             for (int ch = 0; ch < CH; ++ch) v_rgb[ch] = 0.f;
             if (valid) {
@@ -315,17 +319,20 @@ raster_bwd_kernel(const int64_t N, const float* __restrict__ means2d, const floa
                     v_mx = v_sigma * (a * dx + b * dy);
                     v_my = v_sigma * (b * dx + c * dy);
                     v_op = vis * v_alpha;
+                    if constexpr (kAbs) { v_ax = fabsf(v_mx); v_ay = fabsf(v_my); }  // |.| of this pixel's term
                 }
             }
             // spread reduction: lane L ends up with the total of value L >> kShift (colours first, then conic a, b,
-            // c, mean x, y, opacity), and those lanes add it to the gradient arrays in one atomic instruction
-            constexpr int kVals = CH + 6, P = kVals <= 8 ? 8 : 16, kShift = P == 16 ? 1 : 2;
+            // c, mean x, y, opacity[, |mean x|, |mean y|]), and those lanes add it to the gradient arrays in one atomic
+            // instruction
+            constexpr int kVals = CH + (kAbs ? 8 : 6), P = kVals <= 8 ? 8 : 16, kShift = P == 16 ? 1 : 2;
             float v[P];
 #pragma unroll
             for (int q = 0; q < P; ++q) v[q] = 0.0f;
 #pragma unroll
             for (int ch = 0; ch < CH; ++ch) v[ch] = v_rgb[ch];
             v[CH] = v_ca; v[CH + 1] = v_cb; v[CH + 2] = v_cc; v[CH + 3] = v_mx; v[CH + 4] = v_my; v[CH + 5] = v_op;
+            if constexpr (kAbs) { v[CH + 6] = v_ax; v[CH + 7] = v_ay; }
             warp_reduce_spread<P>(v, lane);
             const int which = (int)(lane >> kShift);
             if ((lane & ((1u << kShift) - 1u)) == 0u && which < kVals) {
@@ -334,7 +341,8 @@ raster_bwd_kernel(const int64_t N, const float* __restrict__ means2d, const floa
                 if (which < CH) dst = g_colors + g * CH + which;
                 else if (which < CH + 3) dst = g_conics + 3 * g + (which - CH);
                 else if (which < CH + 5) dst = g_means2d + 2 * g + (which - CH - 3);
-                else dst = g_opac + g;
+                else if (!kAbs || which == CH + 5) dst = g_opac + g;
+                else dst = g_means2d_abs + 2 * g + (which - CH - 6);
                 atomicAdd(dst, v[0]);
             }
           }
@@ -372,13 +380,15 @@ __device__ __forceinline__ float rcp_approx_b(const float x) {
 }
 __device__ __forceinline__ float2 dupb(const float v) { return make_float2(v, v); }
 
+template <bool kAbs>
 __global__ void __launch_bounds__(kBwdThreads)
 raster_bwd_pair_kernel(const int64_t N, const float4* __restrict__ rec, const float* __restrict__ background,
                        const int32_t* __restrict__ tile_ranges, const int32_t* __restrict__ tile_order,
                        const int32_t* __restrict__ sorted_ids, const int W, const int H, const int tiles_w,
                        const float* __restrict__ final_T, const int32_t* __restrict__ last_idx,
                        const float* __restrict__ grad_image, float* __restrict__ g_means2d,
-                       float* __restrict__ g_conics, float* __restrict__ g_colors, float* __restrict__ g_opac) {
+                       float* __restrict__ g_conics, float* __restrict__ g_colors, float* __restrict__ g_opac,
+                       float* __restrict__ g_means2d_abs) {
     __shared__ float4 s_rec[2 * kBwdBatch * kPairRec];
     __shared__ int32_t s_id[2 * kBwdBatch];
     __shared__ int s_max_last;
@@ -444,14 +454,17 @@ raster_bwd_pair_kernel(const int64_t N, const float4* __restrict__ rec, const fl
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
     // loop-invariant roles of the lanes that issue the atomics: lane 4 k adds value k of the spread reduction (colours,
-    // conic a b c, mean x y), lane 1 the opacity gradient -- one predicated RED instruction per Gaussian and warp
+    // conic a b c, mean x y), lane 1 the opacity gradient[, lanes 9 and 17 the absolute mean gradient x and y] -- one
+    // predicated RED instruction per Gaussian and warp
     const int which = lane >> 2;
     const bool role_mean = which >= 6, role_my = which == 7, role_op = lane == 1;
-    const bool issues = ((lane & 3) == 0) || role_op;
+    const bool role_abs = kAbs && (lane == 9 || lane == 17);
+    const bool issues = ((lane & 3) == 0) || role_op || role_abs;
     float* role_base;
     int role_stride;
     float role_scale = 1.0f;
     if (role_op) { role_base = g_opac; role_stride = 1; }
+    else if (role_abs) { role_base = g_means2d_abs + (lane >> 4); role_stride = 2; }
     else if (which < 3) { role_base = g_colors + which; role_stride = 3; }
     else if (which < 6) { role_base = g_conics + (which - 3); role_stride = 3; role_scale = (which == 4) ? 1.0f : 0.5f; }
     else { role_base = g_means2d + (which - 6); role_stride = 2; }
@@ -527,21 +540,34 @@ raster_bwd_pair_kernel(const int64_t N, const float4* __restrict__ rec, const fl
                 v[0] = vr.x + vr.y; v[1] = vg.x + vg.y; v[2] = vb.x + vb.y;
                 v[3] = xx.x + xx.y; v[4] = xy.x + xy.y; v[5] = yy.x + yy.y;
                 v[6] = vsdx.x + vsdx.y; v[7] = vsdy.x + vsdy.y;
-                float ss = vs.x + vs.y;
-                warp_reduce_spread<8>(v, (unsigned)lane);  // lane 4 k holds the total of value k
-#pragma unroll
-                for (int d = 16; d > 0; d >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, d);
-                const float sx = __shfl_sync(0xffffffffu, v[0], 24), sy = __shfl_sync(0xffffffffu, v[0], 28);
-                const int64_t g = lds_i32(a_idc + 4u * (uint32_t)slot);
-                BSPLAT_DASSERT(g >= 0 && g < N);  // (a record that is not a Gaussian never passes the alpha test)
                 // conic of the record: (a, b, c) = (-2 nA, -nB, -2 nC) / log2e;  mean gradient = (a sx + b sy, b sx + c sy)
                 constexpr float kInv = 1.0f / kLog2e;
                 const float cb_ = -kInv * p0.w;
+                float ss = vs.x + vs.y;
+                if constexpr (kAbs) {
+                    // each pixel's own mean gradient v_sigma (a dx + b dy, b dx + c dy), made absolute before any sum;
+                    // reduced together with the opacity's sum: lanes 0-7 get sum v_sigma, 8-15 sum |x|, 16-23 sum |y|
+                    const float ca = -2.0f * kInv * p0.z, cc = -2.0f * kInv * p1.x;
+                    const float2 mx = __ffma2_rn(dupb(ca), vsdx, __fmul2_rn(dupb(cb_), vsdy));
+                    const float2 my = __ffma2_rn(dupb(cb_), vsdx, __fmul2_rn(dupb(cc), vsdy));
+                    float w[4] = {ss, fabsf(mx.x) + fabsf(mx.y), fabsf(my.x) + fabsf(my.y), 0.0f};
+                    warp_reduce_spread<4>(w, (unsigned)lane);
+                    ss = w[0];
+                }
+                warp_reduce_spread<8>(v, (unsigned)lane);  // lane 4 k holds the total of value k
+                if constexpr (!kAbs) {
+#pragma unroll
+                    for (int d = 16; d > 0; d >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, d);
+                }
+                const float sx = __shfl_sync(0xffffffffu, v[0], 24), sy = __shfl_sync(0xffffffffu, v[0], 28);
+                const int64_t g = lds_i32(a_idc + 4u * (uint32_t)slot);
+                BSPLAT_DASSERT(g >= 0 && g < N);  // (a record that is not a Gaussian never passes the alpha test)
                 const float c_first = role_my ? cb_ : -2.0f * kInv * p0.z;
                 const float c_second = role_my ? -2.0f * kInv * p1.x : cb_;
                 float val = role_mean ? (c_first * sx + c_second * sy) : role_scale * v[0];
                 // d alpha / d opacity = alpha / opacity  =>  -sum v_sigma / opacity, opacity = 2^L
                 val = role_op ? -ss * ex2_approx_b(-p1.y) : val;
+                if constexpr (kAbs) val = role_abs ? ss : val;  // lanes 9 and 17 hold sum |x| and sum |y|
                 if (issues) atomicAdd(role_base + g * role_stride, val);
             }
         }
@@ -623,15 +649,14 @@ namespace bsplat {
 int raster_records_launch(int64_t N, const float* means2d, const float* conics, const float* colors,
                           const float* opacities, void* rec_ws, cudaStream_t stream);
 }
-extern "C" int bsplat_rasterize_bwd_fast(int64_t N, const float* means2d, const float* conics, const float* colors,
-                                         const float* opacities, const float* background,
-                                         const int32_t* tile_ranges, const int32_t* tile_order,
-                                         const int32_t* sorted_ids, int64_t M, int32_t width, int32_t height,
-                                         const float* final_T, const int32_t* last_idx, const float* grad_image,
-                                         float* grad_means2d, float* grad_conics, float* grad_colors,
-                                         float* grad_opacities, void* workspace, size_t workspace_bytes,
-                                         void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
+namespace {
+// bsplat_rasterize_bwd_fast[_abs]: g_abs == nullptr launches the plain kernel
+int rasterize_bwd_fast_impl(int64_t N, const float* means2d, const float* conics, const float* colors,
+                            const float* opacities, const float* background, const int32_t* tile_ranges,
+                            const int32_t* tile_order, const int32_t* sorted_ids, int64_t M, int32_t width,
+                            int32_t height, const float* final_T, const int32_t* last_idx, const float* grad_image,
+                            float* grad_means2d, float* grad_conics, float* grad_colors, float* grad_opacities,
+                            float* g_abs, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
     if (N < 0 || M < 0 || !tile_ranges || !background || !final_T || !last_idx || !grad_image) return BSPLAT_E_ARG;
     if (N > 0 && (!grad_means2d || !grad_conics || !grad_colors || !grad_opacities)) return BSPLAT_E_ARG;
     if (M > 0 && (!sorted_ids || !means2d || !conics || !colors || !opacities)) return BSPLAT_E_ARG;
@@ -643,21 +668,26 @@ extern "C" int bsplat_rasterize_bwd_fast(int64_t N, const float* means2d, const 
     const int tiles_w = (width + 15) / 16, tiles_h = (height + 15) / 16;
     int rc = raster_records_launch(N, means2d, conics, colors, opacities, workspace, stream);
     if (rc != BSPLAT_OK) return rc;
-    raster_bwd_pair_kernel<<<(unsigned)(tiles_w * tiles_h), kBwdThreads, 0, stream>>>(
-        N, static_cast<const float4*>(workspace), background, tile_ranges, tile_order, sorted_ids, width, height,
-        tiles_w, final_T, last_idx, grad_image, grad_means2d, grad_conics, grad_colors, grad_opacities);
+    const unsigned grid = (unsigned)(tiles_w * tiles_h);
+    if (g_abs)
+        raster_bwd_pair_kernel<true><<<grid, kBwdThreads, 0, stream>>>(
+            N, static_cast<const float4*>(workspace), background, tile_ranges, tile_order, sorted_ids, width, height,
+            tiles_w, final_T, last_idx, grad_image, grad_means2d, grad_conics, grad_colors, grad_opacities, g_abs);
+    else
+        raster_bwd_pair_kernel<false><<<grid, kBwdThreads, 0, stream>>>(
+            N, static_cast<const float4*>(workspace), background, tile_ranges, tile_order, sorted_ids, width, height,
+            tiles_w, final_T, last_idx, grad_image, grad_means2d, grad_conics, grad_colors, grad_opacities, nullptr);
     BSPLAT_LAUNCH_CHECK();
     return BSPLAT_OK;
 }
 
-extern "C" int bsplat_rasterize_bwd(int64_t N, int32_t channels, const float* means2d, const float* conics,
-                                    const float* colors, const float* opacities, const float* background,
-                                    const int32_t* tile_ranges, const int32_t* sorted_ids, int64_t M,
-                                    int32_t width, int32_t height, int32_t tile_size, const float* final_T,
-                                    const int32_t* last_idx, const float* grad_image, float* grad_means2d,
-                                    float* grad_conics, float* grad_colors, float* grad_opacities,
-                                    void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
+// bsplat_rasterize_bwd[_abs]: g_abs == nullptr launches the plain kernels
+int rasterize_bwd_impl(int64_t N, int32_t channels, const float* means2d, const float* conics, const float* colors,
+                       const float* opacities, const float* background, const int32_t* tile_ranges,
+                       const int32_t* sorted_ids, int64_t M, int32_t width, int32_t height, int32_t tile_size,
+                       const float* final_T, const int32_t* last_idx, const float* grad_image, float* grad_means2d,
+                       float* grad_conics, float* grad_colors, float* grad_opacities, float* g_abs,
+                       cudaStream_t stream) {
     if (N < 0 || M < 0 || !tile_ranges || !background || !final_T || !last_idx || !grad_image) return BSPLAT_E_ARG;
     if (N > 0 && (!grad_means2d || !grad_conics || !grad_colors || !grad_opacities)) return BSPLAT_E_ARG;
     if (M > 0 && (!sorted_ids || !means2d || !conics || !colors || !opacities)) return BSPLAT_E_ARG;
@@ -669,22 +699,84 @@ extern "C" int bsplat_rasterize_bwd(int64_t N, int32_t channels, const float* me
     const int nthreads = round_up32(tile_size * tile_size);
     const dim3 grid(tiles_w, tiles_h);
     const size_t smem = (size_t)nthreads * (10 + channels) * sizeof(float);
-#define BSPLAT_BWD(CH)                                                                                          \
+#define BSPLAT_BWD(CH, ABS)                                                                                     \
     do {                                                                                                        \
         if (smem + 256 > 48 * 1024) /* (+ the kernel's static shared memory) */                                 \
-            BSPLAT_CUDA_TRY(cudaFuncSetAttribute(raster_bwd_kernel<CH>,                                         \
+            BSPLAT_CUDA_TRY(cudaFuncSetAttribute(raster_bwd_kernel<CH, ABS>,                                    \
                                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));      \
-        raster_bwd_kernel<CH><<<grid, nthreads, smem, stream>>>(N, means2d, conics, colors, opacities,         \
+        raster_bwd_kernel<CH, ABS><<<grid, nthreads, smem, stream>>>(N, means2d, conics, colors, opacities,    \
             background, tile_ranges, sorted_ids, width, height, tile_size, tiles_w, final_T, last_idx,          \
-            grad_image, grad_means2d, grad_conics, grad_colors, grad_opacities);                                \
+            grad_image, grad_means2d, grad_conics, grad_colors, grad_opacities, g_abs);                         \
+    } while (0)
+#define BSPLAT_BWD_CH(CH)                 \
+    do {                                  \
+        if (g_abs) BSPLAT_BWD(CH, true);  \
+        else BSPLAT_BWD(CH, false);       \
     } while (0)
     switch (channels) {
-        case 1: BSPLAT_BWD(1); break;
-        case 2: BSPLAT_BWD(2); break;
-        case 3: BSPLAT_BWD(3); break;
-        default: BSPLAT_BWD(4); break;
+        case 1: BSPLAT_BWD_CH(1); break;
+        case 2: BSPLAT_BWD_CH(2); break;
+        case 3: BSPLAT_BWD_CH(3); break;
+        default: BSPLAT_BWD_CH(4); break;
     }
+#undef BSPLAT_BWD_CH
 #undef BSPLAT_BWD
     BSPLAT_LAUNCH_CHECK();
     return BSPLAT_OK;
+}
+}  // namespace
+
+extern "C" int bsplat_rasterize_bwd_fast(int64_t N, const float* means2d, const float* conics, const float* colors,
+                                         const float* opacities, const float* background,
+                                         const int32_t* tile_ranges, const int32_t* tile_order,
+                                         const int32_t* sorted_ids, int64_t M, int32_t width, int32_t height,
+                                         const float* final_T, const int32_t* last_idx, const float* grad_image,
+                                         float* grad_means2d, float* grad_conics, float* grad_colors,
+                                         float* grad_opacities, void* workspace, size_t workspace_bytes,
+                                         void* stream_) {
+    return rasterize_bwd_fast_impl(N, means2d, conics, colors, opacities, background, tile_ranges, tile_order,
+                                   sorted_ids, M, width, height, final_T, last_idx, grad_image, grad_means2d,
+                                   grad_conics, grad_colors, grad_opacities, nullptr, workspace, workspace_bytes,
+                                   (cudaStream_t)stream_);
+}
+
+// ... that also ACCUMULATES, per Gaussian, the sum over pixels of |d loss_p / d means2d| into grad_means2d_abs [N, 2]
+extern "C" int bsplat_rasterize_bwd_fast_abs(int64_t N, const float* means2d, const float* conics,
+                                             const float* colors, const float* opacities, const float* background,
+                                             const int32_t* tile_ranges, const int32_t* tile_order,
+                                             const int32_t* sorted_ids, int64_t M, int32_t width, int32_t height,
+                                             const float* final_T, const int32_t* last_idx, const float* grad_image,
+                                             float* grad_means2d, float* grad_means2d_abs, float* grad_conics,
+                                             float* grad_colors, float* grad_opacities, void* workspace,
+                                             size_t workspace_bytes, void* stream_) {
+    if (N > 0 && !grad_means2d_abs) return BSPLAT_E_ARG;
+    return rasterize_bwd_fast_impl(N, means2d, conics, colors, opacities, background, tile_ranges, tile_order,
+                                   sorted_ids, M, width, height, final_T, last_idx, grad_image, grad_means2d,
+                                   grad_conics, grad_colors, grad_opacities, grad_means2d_abs, workspace,
+                                   workspace_bytes, (cudaStream_t)stream_);
+}
+
+extern "C" int bsplat_rasterize_bwd(int64_t N, int32_t channels, const float* means2d, const float* conics,
+                                    const float* colors, const float* opacities, const float* background,
+                                    const int32_t* tile_ranges, const int32_t* sorted_ids, int64_t M,
+                                    int32_t width, int32_t height, int32_t tile_size, const float* final_T,
+                                    const int32_t* last_idx, const float* grad_image, float* grad_means2d,
+                                    float* grad_conics, float* grad_colors, float* grad_opacities,
+                                    void* stream_) {
+    return rasterize_bwd_impl(N, channels, means2d, conics, colors, opacities, background, tile_ranges, sorted_ids,
+                              M, width, height, tile_size, final_T, last_idx, grad_image, grad_means2d, grad_conics,
+                              grad_colors, grad_opacities, nullptr, (cudaStream_t)stream_);
+}
+
+extern "C" int bsplat_rasterize_bwd_abs(int64_t N, int32_t channels, const float* means2d, const float* conics,
+                                        const float* colors, const float* opacities, const float* background,
+                                        const int32_t* tile_ranges, const int32_t* sorted_ids, int64_t M,
+                                        int32_t width, int32_t height, int32_t tile_size, const float* final_T,
+                                        const int32_t* last_idx, const float* grad_image, float* grad_means2d,
+                                        float* grad_means2d_abs, float* grad_conics, float* grad_colors,
+                                        float* grad_opacities, void* stream_) {
+    if (N > 0 && !grad_means2d_abs) return BSPLAT_E_ARG;
+    return rasterize_bwd_impl(N, channels, means2d, conics, colors, opacities, background, tile_ranges, sorted_ids,
+                              M, width, height, tile_size, final_T, last_idx, grad_image, grad_means2d, grad_conics,
+                              grad_colors, grad_opacities, grad_means2d_abs, (cudaStream_t)stream_);
 }

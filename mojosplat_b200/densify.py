@@ -5,9 +5,10 @@ synchronisation); ``densify_and_prune`` then clones, splits and prunes the Gauss
 read-back of four counts and one gather kernel that writes every parameter and, with ``optimizer``, every Adam moment
 of the new set.  ``scene_extent`` is 3DGS's camera-extent helper.
 
-The other standard recipe, 3DGS-MCMC's relocation and sample-add under a fixed budget, is ``mcmc.py``.  Out of scope
-here: the opacity reset (two torch lines, see ``densify_and_prune``), AbsGS gradients, fused optimizers and multi-GPU
-densification.
+AbsGS's absolute gradients come from the rasterizer backward (``render_gaussians_diff(..., absgrad=True)``) and feed
+``DensifyStats.accumulate`` unchanged.  The other standard recipe, 3DGS-MCMC's relocation and sample-add under a fixed
+budget, is ``mcmc.py``.  Out of scope here: the opacity reset (two torch lines, see ``densify_and_prune``), AbsGS's
+own rules for combining the signed and absolute criteria, fused optimizers and multi-GPU densification.
 """
 from __future__ import annotations
 
@@ -57,7 +58,11 @@ class DensifyStats:
 
     def accumulate(self, means2d_grad: torch.Tensor, radii: torch.Tensor, width: int, height: int) -> None:
         """Add one view: ``means2d_grad`` (N, 2) is d loss / d means2d in pixels (``aux["means2d"].grad`` after
-        ``retain_grad()``), ``radii`` (N, 2) int32 the projection's radii; rows with ``max(radii) == 0`` are skipped."""
+        ``retain_grad()``), ``radii`` (N, 2) int32 the projection's radii; rows with ``max(radii) == 0`` are skipped.
+
+        For AbsGS pass ``aux["means2d_absgrad"]`` of ``render_gaussians_diff(..., absgrad=True, return_aux=True)``
+        instead: the sum over pixels of the absolute per-pixel gradients, which gets the same NDC scaling and norm as
+        gsplat applies to its ``absgrad``; densify on it with gsplat's threshold, ``grad_threshold=0.0008``."""
         _check_cuda_f32("means2d_grad", means2d_grad)
         if means2d_grad.shape != (self.N, 2) or not isinstance(radii, torch.Tensor) or radii.shape != (self.N, 2):
             raise ValueError(f"expected means2d_grad and radii of shape ({self.N}, 2), got "
@@ -145,7 +150,9 @@ def densify_and_prune(params: dict, stats: DensifyStats, scene_extent: float, *,
     an (N, ...) float32 CUDA tensor copied row-wise (opacities, colours, (N, K, 3) SH, ...).  With ``avg = grad2d /
     count`` of ``stats``:
 
-    - ``count > 0`` and ``avg >= grad_threshold``: a Gaussian whose largest log-scale is ``<= log(percent_dense *
+    - ``count > 0`` and ``avg >= grad_threshold`` (2e-4 is 3DGS's value for the signed gradient; statistics of the
+      absolute gradient, ``aux["means2d_absgrad"]``, are used with gsplat's ``0.0008``): a Gaussian whose largest
+      log-scale is ``<= log(percent_dense *
       scene_extent)`` is cloned (the row, then an identical copy), any other is split into two children at
       ``mu + R(q / |q|) (exp(s) * n)``, ``n`` from ``torch.randn((n_split, 2, 3), generator=generator)``, with
       log-scales ``s - ln 1.6``;

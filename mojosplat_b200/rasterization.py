@@ -3,6 +3,8 @@
 ``rasterize_gaussians(means2d, conics, colors, opacities, background_color, tile_ranges,
 sorted_gaussian_indices, camera, tile_size=16, backend)`` -> ``image[H, W, C]`` float32.
 Opacities are used raw (no sigmoid), tile_ranges may be int64 (cast like rasterization.py:163).
+``rasterize_gaussians_diff`` is the differentiable counterpart; with ``means2d_absgrad`` its backward also adds
+AbsGS's absolute screen-space gradients (gsplat's ``absgrad``) into that tensor.
 """
 from __future__ import annotations
 
@@ -113,7 +115,7 @@ class _RasterizeFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, means2d, conics, colors, opacities, background, tile_ranges, sorted_ids, H, W, tile_size,
-                mode="fast"):
+                mode="fast", means2d_absgrad=None):
         L = _lib.require_device(means2d.device)
         dev, means2d, conics, colors, opacities, background, tile_ranges, sorted_ids, N, C = _prep(
             means2d, conics, colors, opacities, background, tile_ranges, sorted_ids)
@@ -150,6 +152,7 @@ class _RasterizeFn(torch.autograd.Function):
         ctx.dims = (H, W, int(tile_size))
         ctx.fast = fast
         ctx.order = order if fast else None  # heavy tiles first: reused by the backward pass
+        ctx.absgrad = means2d_absgrad  # an output of the backward, not an input: added into, never saved
         return image
 
     @staticmethod
@@ -162,35 +165,55 @@ class _RasterizeFn(torch.autograd.Function):
         grad_image = grad_image.to(torch.float32).contiguous()
         g_m = torch.zeros_like(means2d); g_k = torch.zeros_like(conics)
         g_c = torch.zeros_like(colors); g_o = torch.zeros_like(opacities)
+        absgrad = ctx.absgrad
+        name = "bsplat_rasterize_bwd_fast" if ctx.fast else "bsplat_rasterize_bwd"
+        name += "" if absgrad is None else "_abs"
+        # the _abs entry points take the absolute-gradient array right after grad_means2d
+        g_means = [_lib.ptr(g_m)] if absgrad is None else [_lib.ptr(g_m), _lib.ptr(absgrad)]
         with torch.cuda.device(dev):
             if ctx.fast:
                 order = ctx.order
                 ws = _lib.workspace.get(dev, "raster_rec", L.bsplat_rasterize_workspace_bytes(N))
-                rc = L.bsplat_rasterize_bwd_fast(N, _lib.ptr(means2d), _lib.ptr(conics), _lib.ptr(colors),
-                                                 _lib.ptr(opacities), _lib.ptr(background), _lib.ptr(tile_ranges),
-                                                 _lib.ptr(order), _lib.ptr(sorted_ids), sorted_ids.numel(), W, H,
-                                                 _lib.ptr(final_T), _lib.ptr(last_idx), _lib.ptr(grad_image),
-                                                 _lib.ptr(g_m), _lib.ptr(g_k), _lib.ptr(g_c), _lib.ptr(g_o),
-                                                 _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev))
+                rc = getattr(L, name)(N, _lib.ptr(means2d), _lib.ptr(conics), _lib.ptr(colors),
+                                      _lib.ptr(opacities), _lib.ptr(background), _lib.ptr(tile_ranges),
+                                      _lib.ptr(order), _lib.ptr(sorted_ids), sorted_ids.numel(), W, H,
+                                      _lib.ptr(final_T), _lib.ptr(last_idx), _lib.ptr(grad_image), *g_means,
+                                      _lib.ptr(g_k), _lib.ptr(g_c), _lib.ptr(g_o), _lib.ptr(ws), ws.numel(),
+                                      _lib.stream_ptr(dev))
             else:
-                rc = L.bsplat_rasterize_bwd(N, C, _lib.ptr(means2d), _lib.ptr(conics), _lib.ptr(colors),
-                                            _lib.ptr(opacities), _lib.ptr(background), _lib.ptr(tile_ranges),
-                                            _lib.ptr(sorted_ids), sorted_ids.numel(), W, H, ts, _lib.ptr(final_T),
-                                            _lib.ptr(last_idx), _lib.ptr(grad_image), _lib.ptr(g_m), _lib.ptr(g_k),
-                                            _lib.ptr(g_c), _lib.ptr(g_o), _lib.stream_ptr(dev))
-        _lib.check(rc, "bsplat_rasterize_bwd_fast" if ctx.fast else "bsplat_rasterize_bwd")
+                rc = getattr(L, name)(N, C, _lib.ptr(means2d), _lib.ptr(conics), _lib.ptr(colors),
+                                      _lib.ptr(opacities), _lib.ptr(background), _lib.ptr(tile_ranges),
+                                      _lib.ptr(sorted_ids), sorted_ids.numel(), W, H, ts, _lib.ptr(final_T),
+                                      _lib.ptr(last_idx), _lib.ptr(grad_image), *g_means, _lib.ptr(g_k),
+                                      _lib.ptr(g_c), _lib.ptr(g_o), _lib.stream_ptr(dev))
+        _lib.check(rc, name)
         g_bg = (final_T.unsqueeze(-1) * grad_image).sum(dim=(0, 1))
-        return g_m, g_k, g_c, g_o, g_bg, None, None, None, None, None, None
+        return g_m, g_k, g_c, g_o, g_bg, None, None, None, None, None, None, None
 
 
 def rasterize_gaussians_diff(means2d, conics, colors, opacities, background_color, tile_ranges,
-                             sorted_gaussian_indices, camera, tile_size=16, mode="fast"):
+                             sorted_gaussian_indices, camera, tile_size=16, mode="fast", means2d_absgrad=None):
     """Differentiable ``rasterize_gaussians`` (additive: the reference is forward-only, render.py:11).
     Gradients flow to means2d, conics, colors, opacities and background_color; the tile lists are
     treated as constants. Forward values: ``mode="fast"`` (16x16 tiles, RGB) = the default inference kernel's, bit for
-    bit; ``mode="faithful"`` (and every other shape) = the faithful kernel's."""
+    bit; ``mode="faithful"`` (and every other shape) = the faithful kernel's.
+
+    ``means2d_absgrad``: an optional (N, 2) float32 contiguous tensor on means2d's device.  Every backward pass through
+    this image ADDS to it, per Gaussian, the sum over the pixels it was composited at of |d loss_p / d means2d| (x and
+    y separately, the absolute value taken per pixel): AbsGS's densification statistic, gsplat's ``absgrad``.  Unlike
+    the signed gradient it does not cancel when pixels on opposite sides pull the mean in opposite directions."""
     if mode not in ("fast", "faithful"):
         raise ValueError(f"Invalid mode: {mode}")
+    if means2d_absgrad is not None:
+        N = means2d.shape[0]
+        if not isinstance(means2d_absgrad, torch.Tensor) or means2d_absgrad.shape != (N, 2):
+            raise ValueError(f"means2d_absgrad must be a ({N}, 2) tensor, got "
+                             f"{tuple(getattr(means2d_absgrad, 'shape', ()))}")
+        if means2d_absgrad.dtype != torch.float32 or not means2d_absgrad.is_contiguous():
+            raise ValueError(f"means2d_absgrad must be contiguous float32, got {means2d_absgrad.dtype}")
+        if means2d_absgrad.device != means2d.device:
+            raise ValueError(f"means2d_absgrad is on {means2d_absgrad.device}, means2d on {means2d.device}")
     opac = opacities.reshape(-1)
     return _RasterizeFn.apply(means2d, conics, colors, opac, background_color, tile_ranges,
-                              sorted_gaussian_indices, int(camera.H), int(camera.W), int(tile_size), mode)
+                              sorted_gaussian_indices, int(camera.H), int(camera.W), int(tile_size), mode,
+                              means2d_absgrad)

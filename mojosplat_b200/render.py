@@ -6,7 +6,8 @@ intersects :73-76, ``sh_degree`` accepted but only truncating features :82-87). 
 backend the three stages run inside ONE C call (bsplat_render_fwd): projection -> count+scan ->
 one 32-byte read-back (M, depth-key range) -> emit -> onesweep sort -> tile ranges -> raster, all
 on the caller's current stream, workspace reused across frames.
-``render_gaussians_diff`` is the differentiable counterpart (stage by stage, with autograd).
+``render_gaussians_diff`` is the differentiable counterpart (stage by stage, with autograd); with ``absgrad=True``
+it also collects AbsGS's absolute screen-space gradients for densification.
 """
 from __future__ import annotations
 
@@ -98,6 +99,7 @@ def render_gaussians_diff(
     tile_size: int = TILE_SIZE,
     backend: str = "cuda",
     return_aux: bool = False,
+    absgrad: bool = False,
 ):
     """Differentiable ``render_gaussians``: image (H, W, C) with gradients for means3d, the log-scales, the raw quats,
     opacities, features (colours or SH coefficients) and a background_color tensor.  Arguments, checks and the
@@ -111,7 +113,14 @@ def render_gaussians_diff(
 
     ``return_aux=True`` also returns ``dict(means2d, radii, depths, conics, tile_ranges, sorted_ids)``; ``means2d`` is
     the tensor of the graph (``retain_grad()`` it for screen-space statistics) and ``radii > 0`` marks the visible
-    Gaussians."""
+    Gaussians.
+
+    ``absgrad=True`` (needs ``return_aux=True``) adds ``aux["means2d_absgrad"]``, a zero (N, 2) float32 tensor that
+    every backward pass through the image adds to: per Gaussian, the sum over the pixels it was composited at of
+    |d loss_p / d means2d| (AbsGS; gsplat's ``info["means2d"].absgrad``).  It stays zero when no Gaussian overlaps a
+    tile.  Densify on it with ``DensifyStats.accumulate(aux["means2d_absgrad"], aux["radii"], W, H)``."""
+    if absgrad and not return_aux:
+        raise ValueError("absgrad=True returns its statistic in aux: pass return_aux=True")
     required = [means3d, scales, quats, opacities, features]
     if not all(isinstance(t, torch.Tensor) and t.is_cuda for t in required):
         raise ValueError("All input gaussian tensors must be CUDA tensors.")
@@ -137,16 +146,19 @@ def render_gaussians_diff(
     means2d, conics, depths, radii = project_gaussians_diff(means3d, scales, quats, opacities, camera, backend)
     sorted_ids, tile_ranges = bin_gaussians_to_tiles_cuda(means2d.detach(), radii, depths.detach(), H, W,
                                                           tile_size, semantics=CUDA_BACKENDS[backend])
+    extra = {}
+    if absgrad:
+        extra["means2d_absgrad"] = torch.zeros((means2d.shape[0], 2), dtype=torch.float32, device=means2d.device)
     if sorted_ids.numel() == 0:
         warnings.warn("No Gaussian overlaps found; returning the background")
         image = bg.to(torch.float32).expand(H, W, bg.shape[0]).clone()
     else:
         image = rasterize_gaussians_diff(means2d, conics, colors, opacities, bg, tile_ranges, sorted_ids, camera,
-                                         tile_size)
+                                         tile_size, means2d_absgrad=extra.get("means2d_absgrad"))
     image = image.to(features.dtype)
     if return_aux:
         return image, dict(means2d=means2d, radii=radii, depths=depths, conics=conics, tile_ranges=tile_ranges,
-                           sorted_ids=sorted_ids)
+                           sorted_ids=sorted_ids, **extra)
     return image
 
 
